@@ -20,6 +20,10 @@ collective is on this path).  Prints ONE JSON line on rank 0.
   cpu_baseline  the reference's CPU path (installed torchaudio wheel, hot-path source identical to
             /root/reference) or, if that cannot be imported, the numpy oracle port -- rank 0, N = 1 only
   --impl reference   the same reference CPU path as its own arm: the FULL 256 x 160000 batch per step
+  --dump-outputs DIR  after the timing, rank 0 writes what the LAST timed step of each GPU section returned, as float32
+            DIR/<name>.npy: the headline MelSpectrogram in full, and of the other configs a fixed seeded sample of whole
+            rows (at most DUMP_SIDE_BYTES each); the e2e result is asserted equal to the headline's.  Inputs come from
+            seeded generators, so two builds run with the same arguments can be compared output for output.
 """
 import argparse
 import json
@@ -47,6 +51,8 @@ ALGO_BYTES = 4 * (BATCH * LENGTH + BATCH * FRAMES * N_MELS) + 4 * (N_FFT + (N_FF
 # the write-back of part of the 51 MB output is still in L2 at kernel end
 NCU_DRAM_BYTES = 196_650_752
 NCU_DRAM_SOURCE = "ncu --set full, profiles/r2_mel_v3_tc2_prefetch.txt (dram read 163.99 MB + write 32.66 MB per launch)"
+DUMP_BYTES = 64 << 20  # --dump-outputs: every array together (the headline alone is 51.3 MB)
+DUMP_SIDE_BYTES = 2 << 20  # --dump-outputs: each array of the other configs
 
 
 def workload_config(world):
@@ -54,6 +60,30 @@ def workload_config(world):
     return {"workload": WORKLOAD, "global_batch": world * BATCH, "frames_per_step": world * BATCH * FRAMES,
             "parallelism": f"batch shard x{world}, no collective",
             "l2": "input 163.8 MB per step > 126 MB L2 (no flush needed)"}
+
+
+def dump_array(t, max_bytes=None):
+    """`t` as a contiguous float32 host array; above `max_bytes`, only the whole rows (dim 0) of a fixed seeded choice
+    that fit, in ascending order, so every run of the same arguments samples the same rows."""
+    import numpy as np
+    import torch
+
+    rows = t.shape[0]
+    keep = rows if max_bytes is None else max(1, min(rows, max_bytes // (4 * t[0].numel())))
+    if keep < rows:
+        idx = np.sort(np.random.default_rng(0).choice(rows, keep, replace=False))
+        t = t[torch.from_numpy(idx).to(t.device)]
+    return np.ascontiguousarray(t.float().cpu().numpy())
+
+
+def write_dumps(out_dir, arrays):
+    import numpy as np
+
+    total = sum(a.nbytes for a in arrays.values())
+    assert total <= DUMP_BYTES, f"--dump-outputs would write {total} bytes (limit {DUMP_BYTES})"
+    os.makedirs(out_dir, exist_ok=True)
+    for name, a in arrays.items():
+        np.save(os.path.join(out_dir, f"{name}.npy"), a)
 
 
 def measured_peaks():
@@ -295,17 +325,25 @@ def run_b200(args):
     K, W = args.steps, max(args.warmup, 3)
 
     def time_steps(fn, steps=K, warm=W):
-        """ms per step: `warm` untimed steps, then `steps` steps between two CUDA events, barrier + sync on both sides."""
+        """(ms per step, what the last step returned): `warm` untimed steps, then `steps` steps between two CUDA events,
+        barrier + sync on both sides."""
         for _ in range(warm):
             fn()
         barrier()
         e0, e1 = torch.cuda.Event(enable_timing=True), torch.cuda.Event(enable_timing=True)
         e0.record()
-        for _ in range(steps):
+        for _ in range(steps - 1):
             fn()
+        out = fn()  # outside the loop: keeping every output there would hold it alive across the next step
         e1.record()
         barrier()
-        return e0.elapsed_time(e1) / steps
+        return e0.elapsed_time(e1) / steps, out
+
+    dumps = {}
+
+    def keep(name, out, max_bytes=DUMP_SIDE_BYTES):
+        if args.dump_outputs and rank == 0:
+            dumps[name] = dump_array(out, max_bytes)
 
     def max_over_ranks(values):
         t = torch.tensor(values, device=dev, dtype=torch.float64)
@@ -322,8 +360,8 @@ def run_b200(args):
     # rank 0 samples the clocks of every GPU of the job (local ranks 0 .. world - 1 on this one node)
     with torch.inference_mode(), ClockSampler([local] if world == 1 else range(world), active=(rank == 0)) as clocks:
         # ---- headline: config 2, inputs resident -------------------------------------------------------------
-        ms_step = time_steps(lambda: mel(x))
-        y = mel(x)
+        ms_step, y = time_steps(lambda: mel(x))
+        keep("melspectrogram", y, max_bytes=None)
 
         # ---- end to end: pinned host -> device, fused kernel, device -> pinned host ----------------------------
         from audio_b200.pipeline import HostPipeline
@@ -365,9 +403,11 @@ def run_b200(args):
         mf = T.MFCC(SAMPLE_RATE, n_mfcc=N_MFCC, melkwargs=dict(n_fft=N_FFT, hop_length=HOP, n_mels=N_MELS)).to(dev)
         if world > 1:
             mf.process_group = dist.group.WORLD
-        ms_c4 = time_steps(lambda: mf(x))
+        ms_c4, c4_out = time_steps(lambda: mf(x))
+        keep("mfcc", c4_out)
+        del c4_out
         mf_local = T.MFCC(SAMPLE_RATE, n_mfcc=N_MFCC, melkwargs=dict(n_fft=N_FFT, hop_length=HOP, n_mels=N_MELS)).to(dev)
-        ms_c4_local = time_steps(lambda: mf_local(x)) if world > 1 else ms_c4
+        ms_c4_local = time_steps(lambda: mf_local(x))[0] if world > 1 else ms_c4
         c4_bytes = 4 * (BATCH * LENGTH + BATCH * FRAMES * N_MFCC) + 4 * (N_FFT + 513 * N_MELS + N_MELS * N_MFCC)
         del mf, mf_local
 
@@ -379,7 +419,12 @@ def run_b200(args):
             with warnings.catch_warnings():
                 warnings.simplefilter("ignore")  # n_fft = 256 leaves two of the 80 mel filters empty (reference warns too)
                 m5 = T.MelSpectrogram(SAMPLE_RATE, n_fft=n_fft, hop_length=hop, n_mels=N_MELS).to(dev)
-            ms5 = ms_step if n_fft == N_FFT else time_steps(lambda: m5(x))
+            if n_fft == N_FFT:
+                ms5 = ms_step  # the headline, dumped above
+            else:
+                ms5, out5 = time_steps(lambda: m5(x))
+                keep(f"melspectrogram_nfft{n_fft}", out5)
+                del out5
             sweep.append((n_fft, hop, fr, ms5, 4 * (BATCH * LENGTH + BATCH * fr * N_MELS) + 4 * (n_fft + (n_fft // 2 + 1) * N_MELS)))
             del m5
         del x, y
@@ -388,11 +433,14 @@ def run_b200(args):
         # ---- C3: Resample 44.1 -> 16 kHz, 1024 x 220500 per GPU ------------------------------------------------------
         rs = T.Resample(RS_ORIG, RS_NEW, resampling_method="sinc_interp_kaiser").to(dev)
         xr = torch.randn(RS_ROWS, RS_LEN, device=dev, generator=g)
-        ms_c3 = time_steps(lambda: rs(xr))
+        ms_c3, c3_out = time_steps(lambda: rs(xr))
+        keep("resample", c3_out)
         c3_bytes = 4 * (RS_ROWS * RS_LEN + RS_ROWS * RS_OUT) + 4 * 160 * 475
-        del xr, rs
+        del xr, rs, c3_out
         torch.cuda.empty_cache()
     clock_summary = clocks.summary()
+    if dumps:
+        write_dumps(args.dump_outputs, dumps)
 
     vals = [ms_step, ms_e2e, ms_c4, ms_c4_local, ms_c3] + [s[3] for s in sweep]
     vals = max_over_ranks(vals)
@@ -462,7 +510,13 @@ def main():
     ap.add_argument("--steps", type=int, default=100)
     ap.add_argument("--warmup", type=int, default=5)
     ap.add_argument("--impl", default="b200", choices=["b200", "reference"])
+    ap.add_argument("--dump-outputs", metavar="DIR",
+                    help="write what the last timed step of each GPU section returned to DIR/<name>.npy (float32)")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if args.dump_outputs and args.impl == "reference":
+        ap.error("--dump-outputs records the GPU sections; the reference arm has none")
     if args.impl == "reference":
         run_reference(args)
     else:

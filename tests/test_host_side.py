@@ -311,6 +311,34 @@ def test_bench_clock_sampler_pause_and_fallback():
     assert bench.workload_config(8)["global_batch"] == 8 * bench.BATCH
 
 
+def test_bench_dump_outputs_and_steps(tmp_path):
+    """`bench.py --dump-outputs`: float32 host arrays, the whole tensor when it fits, otherwise the same seeded rows on
+    every run (so two builds can be compared array for array), and a hard cap on what it writes; `--steps` below 1 is
+    refused instead of timing nothing."""
+    import importlib.util
+    import subprocess
+    import sys
+
+    spec = importlib.util.spec_from_file_location("bench_under_test", os.path.join(ROOT, "bench.py"))
+    bench = importlib.util.module_from_spec(spec)
+    spec.loader.exec_module(bench)
+    t = torch.arange(1024 * 3, dtype=torch.float64).reshape(1024, 3)
+    full = bench.dump_array(t)
+    assert full.dtype == np.float32 and np.array_equal(full, t.numpy())
+    a, b = bench.dump_array(t, 6 * 3 * 4), bench.dump_array(t, 6 * 3 * 4)
+    assert a.dtype == np.float32 and a.shape == (6, 3) and np.array_equal(a, b)
+    rows = a[:, 0] / 3
+    assert np.all(np.diff(rows) > 0) and np.array_equal(a, t.numpy()[rows.astype(int)])
+    assert bench.dump_array(t[:, None, :], 1).shape == (1, 1, 3)  # never less than one whole row
+    bench.write_dumps(str(tmp_path / "d"), {"x": a})
+    assert np.array_equal(np.load(tmp_path / "d" / "x.npy"), a)
+    with pytest.raises(AssertionError, match="--dump-outputs"):
+        bench.write_dumps(str(tmp_path / "big"), {"x": np.zeros(bench.DUMP_BYTES // 4 + 1, np.float32)})
+    assert not (tmp_path / "big").exists()
+    proc = subprocess.run([sys.executable, os.path.join(ROOT, "bench.py"), "--steps", "0"], capture_output=True, text=True)
+    assert proc.returncode == 2 and "--steps" in proc.stderr
+
+
 @pytest.mark.parametrize("method", ["sinc_interp_hann", "sinc_interp_kaiser"])
 def test_resample_tc_band_covers_the_reference_kernels_support(method):
     """The tcgen05 resampler's banded plan is computed on the host from (orig', new', width) alone and assumes that
