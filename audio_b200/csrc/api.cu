@@ -37,6 +37,9 @@ int resample_run_impl(const void*, const float*, int, int, int, const float*, in
 
 using namespace b200a;
 
+// complex64 data (and the (sum, count) pairs of b200a_ratio_f32) are read and written as float2: 8-byte alignment
+static bool misaligned8(const void* p) { return (reinterpret_cast<uintptr_t>(p) & 7) != 0; }
+
 #pragma GCC visibility push(default)
 extern "C" {
 
@@ -135,6 +138,7 @@ int b200a_frontend_run(const b200a_frontend_desc* desc, const void* workspace, i
   if (workspace == nullptr || wave == nullptr || out == nullptr) return B200A_EINVAL;
   if (rows < 0 || length < 0 || row_stride < length) return B200A_EINVAL;
   if (stage < B200A_STAGE_COMPLEX || stage > B200A_STAGE_FEAT) return B200A_EINVAL;
+  if (stage == B200A_STAGE_COMPLEX && misaligned8(out)) return B200A_EINVAL;
   if (stage >= B200A_STAGE_MEL && desc->n_mels <= 0) return B200A_EINVAL;
   if (stage != B200A_STAGE_COMPLEX && !(desc->power > 0.f)) return B200A_EINVAL;
   const int64_t ext = length + 2 * (int64_t)desc->pad;
@@ -191,6 +195,7 @@ int b200a_istft_run(const b200a_frontend_desc* desc, const void* workspace, cons
   if (rows < 0 || frames < 1 || out_len < 0 || start < 0 || out_row_stride < out_len) return B200A_EINVAL;
   if (rows == 0 || out_len == 0) return B200A_OK;
   if (workspace == nullptr || spec == nullptr || frame_buf == nullptr || out == nullptr) return B200A_EINVAL;
+  if (misaligned8(spec)) return B200A_EINVAL;
   return istft_run_impl(desc, workspace, spec, rows, frames, stride_row, stride_bin, stride_frame, frame_buf, out,
                         out_row_stride, start, out_len, static_cast<cudaStream_t>(stream));
 }
@@ -201,6 +206,7 @@ int b200a_griffinlim_update(const float* mag, int64_t stride_row, int64_t stride
   if (rows < 0 || bins < 1 || frames < 1 || !(inv_power > 0.f)) return B200A_EINVAL;
   if (rows == 0) return B200A_OK;
   if (mag == nullptr || proj == nullptr || (tprev != nullptr && rebuilt == nullptr)) return B200A_EINVAL;
+  if (misaligned8(proj) || misaligned8(rebuilt) || misaligned8(tprev)) return B200A_EINVAL;
   return griffinlim_update_impl(mag, stride_row, stride_bin, stride_frame, inv_power, rebuilt, tprev, momentum, normalize,
                                 proj, rows, bins, frames, static_cast<cudaStream_t>(stream));
 }
@@ -211,6 +217,7 @@ int b200a_phase_vocoder(const float* spec, int64_t stride_row, int64_t stride_bi
   if (rows < 0 || bins < 1 || frames_in < 1 || frames_out < 0 || !(rate > 0.0)) return B200A_EINVAL;
   if (rows == 0 || frames_out == 0) return B200A_OK;
   if (spec == nullptr || phase_advance == nullptr || out == nullptr) return B200A_EINVAL;
+  if (misaligned8(spec) || misaligned8(out)) return B200A_EINVAL;
   return phase_vocoder_impl(spec, stride_row, stride_bin, stride_frame, rows, bins, frames_in, rate, phase_advance, out,
                             frames_out, static_cast<cudaStream_t>(stream));
 }
@@ -263,7 +270,7 @@ int b200a_subtract_column_mean(float* x, int64_t rows, int64_t frames, int64_t w
 int b200a_ratio_f32(const float* pairs, int64_t n, float* out, b200a_stream stream) {
   if (n < 0) return B200A_EINVAL;
   if (n == 0) return B200A_OK;
-  if (pairs == nullptr || out == nullptr) return B200A_EINVAL;
+  if (pairs == nullptr || out == nullptr || misaligned8(pairs)) return B200A_EINVAL;
   return ratio_impl(pairs, n, out, static_cast<cudaStream_t>(stream));
 }
 

@@ -464,7 +464,7 @@ mfcc_finish_tiled_kernel(const float* __restrict__ feat, int64_t total_rows, int
       s_floor[threadIdx.x] =
           clamp ? group_max[((r0 + threadIdx.x) / frames) / rows_per_group] - top_db : -CUDART_INF_F;
     __syncthreads();
-    if ((n_mels & 3) == 0) {
+    if ((n_mels & 3) == 0 && (reinterpret_cast<uintptr_t>(feat) & 15) == 0) {
       const int q4 = n_mels >> 2;  // float4 per row
       const float4* src = reinterpret_cast<const float4*>(feat + r0 * n_mels);
       for (int i = threadIdx.x; i < rows * q4; i += blockDim.x) {

@@ -231,6 +231,7 @@ struct RsParams {
   int frag_smem_bytes;      // shared memory granted to the fragment copy (0: read them from global)
   int row_spread;           // 1, 2 or 4: frame distance of the 8 rows one A-fragment load touches
   int skip_if_r3_ok;        // launched behind resample_r3_kernel (1) / resample_tc_kernel (2): leave when the header says that kernel did the work
+  int out_pair;             // new' and the row pitch are even and `out` is 8-byte aligned: phase pairs are one float2 store
 };
 
 // Fill one staging buffer with the samples frames [f0, f0 + 32) of `row` need:
@@ -415,7 +416,7 @@ __global__ void __launch_bounds__(kRsMaxWarps * 32, 1) resample_mma_kernel(const
       else contract(std::false_type{});
       // D rows = frames; columns 2c, 2c+1 = phases 8t + 2c (+1): out index = f*new' + phase
       const int j0 = 8 * t + 2 * c;
-      const bool pair_ok = j0 + 1 < p.new_r && (p.new_r & 1) == 0 && (p.out_row_stride & 1) == 0;
+      const bool pair_ok = j0 + 1 < p.new_r && p.out_pair != 0;
 #pragma unroll
       for (int h = 0; h < 2; ++h)
 #pragma unroll
@@ -424,7 +425,7 @@ __global__ void __launch_bounds__(kRsMaxWarps * 32, 1) resample_mma_kernel(const
           const float v1 = d[h][0][2 * half_row + 1] + (d[h][1][2 * half_row + 1] + d[h][2][2 * half_row + 1]);
           const int64_t m = (f0 + fr[2 * h + half_row]) * p.new_r + j0;
           if (pair_ok && m + 1 < p.out_len) {
-            *reinterpret_cast<float2*>(orow + m) = make_float2(v0, v1);  // m even, row pitch even: 8-byte aligned
+            *reinterpret_cast<float2*>(orow + m) = make_float2(v0, v1);  // m even, row pitch even, out aligned: 8 bytes
           } else {
             if (j0 < p.new_r && m < p.out_len) orow[m] = v0;
             if (j0 + 1 < p.new_r && m + 1 < p.out_len) orow[m + 1] = v1;
@@ -1783,6 +1784,7 @@ int resample_run_impl(const void* ws, const float* kernel, int orig_r, int new_r
     }
     p.row_spread = best_spread;
     p.skip_if_r3_ok = r3_launched ? 1 : (tc_launched ? 2 : 0);
+    p.out_pair = (new_r % 2 == 0 && out_row_stride % 2 == 0 && (reinterpret_cast<uintptr_t>(out) & 7) == 0) ? 1 : 0;
     // warps: n_tiles items (phase groups) per tile; prefer the largest count that divides them evenly
     const int items = n_tiles;
     int warps = 8;

@@ -13,7 +13,10 @@
  * No torch/ATen type crosses this boundary: plain pointers, sizes and one POD descriptor.
  *
  * Rules for every function taking a stream:
- *   - all data pointers are DEVICE pointers on the current device, 4-byte aligned, fp32 unless noted;
+ *   - all data pointers are DEVICE pointers on the current device, fp32 unless noted, and 4-byte aligned;
+ *     complex64 buffers (marked "8-byte aligned" below) are read and written as float2 and must be 8-byte
+ *     aligned -- a misaligned one is B200A_EINVAL, before anything is enqueued.  Every other buffer may sit at
+ *     any float offset; kernels that vectorise check the alignment of the pointer they were given;
  *   - the library never allocates, frees or copies device memory behind the caller's back, and
  *     keeps no mutable global state except one-time cudaFuncSetAttribute calls;
  *   - calls are asynchronous; return value 0 (B200A_OK) means "enqueued", a negative value is
@@ -136,7 +139,7 @@ int b200a_frontend_prepare(const b200a_frontend_desc* desc, const float* window,
  * (_transforms.py:403-415)] [+ the dB/log step of MFCC.forward (_transforms.py:701-705)].
  *   wave        : [rows] utterances of `length` samples, row r at wave + r*row_stride
  *   stage       : enum b200a_stage
- *   out         : [rows][T][n_bins] (POWER), [rows][T][n_bins][2] (COMPLEX), [rows][T][n_mels] (MEL/FEAT)
+ *   out         : [rows][T][n_bins] (POWER), [rows][T][n_bins][2] (COMPLEX, 8-byte aligned), [rows][T][n_mels] (MEL/FEAT)
  *   group_max   : FEAT only, may be NULL: [ceil(rows/rows_per_group)] running maxima of the dB
  *                 features, combined with atomic max -- the caller initialises them to -inf
  *                 (b200a_fill_f32).  This is the `amax` of functional.py:399; rows_per_group
@@ -179,7 +182,7 @@ int b200a_amplitude_to_db(const float* x, int64_t groups, int64_t group_elems, f
 int b200a_fill_f32(float* dst, int64_t n, float value, b200a_stream stream);
 
 /*
- * out[i] = pairs[i][0] / pairs[i][1].  Last step of F.spectral_centroid (functional.py:1257-1299): the
+ * out[i] = pairs[i][0] / pairs[i][1]; `pairs` 8-byte aligned.  Last step of F.spectral_centroid (functional.py:1257-1299): the
  * fused front end is run with the two-column "filterbank" [bin frequency | 1] on the magnitude
  * spectrogram, which yields (sum_k f_k |X_k|, sum_k |X_k|) per frame; this divides them.
  */
@@ -192,7 +195,7 @@ int b200a_ratio_f32(const float* pairs, int64_t n, float* out, b200a_stream stre
  * overlap-added squared window, for the output positions [start, start + out_len) of the n_fft + hop*(frames-1)
  * long signal (start = n_fft/2 when center).  The workspace is the one b200a_frontend_prepare built for the same
  * descriptor (window, twiddles, normalisation: `normalized` modes are undone here).  onesided descriptors only.
- *   spec      : complex64, logical [rows][n_fft/2+1][frames], strides in complex elements
+ *   spec      : complex64, logical [rows][n_fft/2+1][frames], strides in complex elements, 8-byte aligned
  *   frame_buf : caller-owned scratch of rows * frames * n_fft floats (the windowed time frames)
  *   out       : [rows] signals of out_len samples, row r at out + r*out_row_stride
  * The caller checks the window envelope (NOLA) -- torch raises when its minimum is < 1e-11; this library divides.
@@ -209,7 +212,7 @@ int b200a_istft_run(const b200a_frontend_desc* desc, const void* workspace, cons
  * angles = rebuilt as is when normalize == 0 (the first inversion with a random initial phase, :310-311).
  *   mag                   : |X|^power, logical [rows][bins][frames] with element strides (the user's tensor)
  *   rebuilt, tprev, proj  : complex64 frame-major [rows][frames][bins] (what b200a_frontend_run(COMPLEX) writes and
- *                           b200a_istft_run reads with strides (frames*bins, 1, bins))
+ *                           b200a_istft_run reads with strides (frames*bins, 1, bins)), 8-byte aligned
  */
 int b200a_griffinlim_update(const float* mag, int64_t stride_row, int64_t stride_bin, int64_t stride_frame,
                             float inv_power, const float* rebuilt, const float* tprev, float momentum,
@@ -220,9 +223,9 @@ int b200a_griffinlim_update(const float* mag, int64_t stride_row, int64_t stride
  * F.phase_vocoder (functional/functional.py:713-803): time-stretch a complex spectrogram by `rate` without changing
  * pitch.  Output frame t' interpolates the magnitudes of input frames trunc(ts), trunc(ts + 1), ts = float(rate * t'),
  * and carries the accumulated phase advance; frames_out = ceil(frames_in / rate) (torch.arange(0, frames_in, rate)).
- *   spec          : complex64, logical [rows][bins][frames_in], strides in complex elements
+ *   spec          : complex64, logical [rows][bins][frames_in], strides in complex elements, 8-byte aligned
  *   phase_advance : [bins] expected phase advance per hop (linspace(0, pi * hop, bins))
- *   out           : complex64 frame-major [rows][frames_out][bins]
+ *   out           : complex64 frame-major [rows][frames_out][bins], 8-byte aligned
  */
 int b200a_phase_vocoder(const float* spec, int64_t stride_row, int64_t stride_bin, int64_t stride_frame, int64_t rows,
                         int64_t bins, int64_t frames_in, double rate, const float* phase_advance, float* out,
