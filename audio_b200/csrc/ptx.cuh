@@ -20,10 +20,6 @@ __device__ __forceinline__ void bulk_g2s(void* dst, const void* src, uint32_t by
                "l"(src), "r"(bytes), "r"(smem_u32(bar))
                : "memory");
 }
-// hint: bring [src, src + bytes) (16-byte aligned, multiple of 16) into L2; no completion tracking
-__device__ __forceinline__ void bulk_prefetch_l2(const void* src, uint32_t bytes) {
-  asm volatile("cp.async.bulk.prefetch.L2.global [%0], %1;" ::"l"(src), "r"(bytes) : "memory");
-}
 // Bounded wait: a mis-programmed copy traps instead of hanging the GPU.  `try_wait` suspends the warp
 // in hardware up to the hinted time, so a waiting warp costs (almost) no issue slots.
 template <uint32_t SUSPEND_NS = 2000>

@@ -6,34 +6,33 @@
 // (numerically) zero: row j only has a contiguous run of ~2*lowpass_width*orig'/min(orig',new')
 // taps around the position of output phase j.
 //
-// Main kernel (resample_mma_kernel): the sum IS a banded matrix product
+// The sum IS a banded matrix product
 //     Y[f][j] = sum_i X[f][i] * K[j][i],   X[f][i] = x[f*orig' + i - width]  (a strided view of the signal)
-// so a CTA stages the samples of 32 output frames in shared memory with one bulk asynchronous copy
-// (double buffered: the next tile lands while this one is multiplied), and its 8 warps run
-// mma.sync.m16n8k8 TF32 tiles of 16 frames x 8 phases over just the k-steps where those 8 phases have
-// live taps, with error-compensated operands (X_hi*K_hi + X_lo*K_hi + X_hi*K_lo, ~2^-21 relative).
-// No padded copy of the input, no (rows, new', frames) intermediate; the output is written already
-// interleaved and truncated.  Each input sample is read from HBM once, each output written once.
+// and three kernel families compute it.  rs_choose picks one from the ratio alone, never from the batch, so a row's
+// result does not depend on what it is batched with; resample_run_impl adds only the per-call conditions (pointer
+// alignment, the 2^31 index bound).
 //
-// Fallback (resample_direct_kernel): one output per thread over the phase's live taps, for ratios whose
-// tables or tiles do not fit (new' > 1024, orig' > ~1100) or mis-aligned inputs.
+// resample_tc_kernel (odd orig', when the banded tcgen05 plan fits: new' <= 160, <= 30 16-tap k-steps, tap blocks
+// in shared memory): convert warps build a K-major bf16 hi / lo operand per 32-frame tile, one thread issues
+// tcgen05.mma over the phases with live taps in each k-step (bf16 x 3, FP32 accumulate).  The plan is computed on the
+// host from (orig', new', width); the device checks it against the measured support of the caller's kernel, and if a
+// tap lies outside the band the kernel leaves and resample_mma_kernel, always launched behind it, does the work.
 //
-// Preferred kernel for odd orig' (resample_simt_kernel, e.g. 44.1 -> 16 kHz): the pruned FIR is only ~68 flop per
-// output sample, far below what keeps the legacy tensor path busy with error-compensated TF32 (3 MMAs per tile,
-// "math pipe throttle" in profiles/r1_resample_v4.txt), so it runs as a register-tiled FP32 product on packed
-// FFMA2 instead: a thread owns ONE frame of each of two adjacent 32-frame half-chunks x a group of 8 phases,
-// lanes are consecutive frames (stride orig' words: conflict-free for odd orig'), the 8 taps of a step are one
-// 32-byte broadcast read, and the two frames ride in the two halves of an f32x2 register pair:
-//     acc[q] (frame a | frame b) += (x_a[i] | x_b[i]) * tap[q][i]      (FFMA2 with a scalar-broadcast operand)
-// Half-chunks stream through a 3-slot ring of bulk asynchronous copies.  Step s pairs half-chunks (s-1, s) and
-// handles the phase groups of parity s & 1, so every half-chunk meets both parities (once as the newer, once as
-// the older member of a pair) and a slot is free for the next copy as soon as its second step ends.
-#include <cstdio>
-#include <cstdlib>
+// resample_mma_kernel (even orig', or odd orig' beyond the tcgen05 limits, while new' <= 1024 and two staging
+// buffers fit): a CTA stages the samples of 32 output frames in shared memory with one bulk asynchronous copy
+// (double buffered: the next tile lands while this one is multiplied), and its warps run mma.sync.m16n8k8 TF32 tiles
+// of 16 frames x 8 phases over just the k-steps where those 8 phases have live taps, with error-compensated operands
+// (X_hi*K_hi + X_lo*K_hi + X_hi*K_lo, ~2^-21 relative).
+//
+// resample_direct_kernel: one output per thread over the phase's live taps, for ratios whose tiles do not fit
+// (new' > 1024, or orig' so large that two 32-frame staging buffers exceed shared memory) and for inputs that are not
+// 4-byte aligned.
+//
+// No padded copy of the input, no (rows, new', frames) intermediate; the output is written already interleaved and
+// truncated.  The two tensor-core kernels read each input sample from HBM once and write each output once.
 #include <type_traits>
 
 #include "common.cuh"
-#include "f32x2.cuh"
 #include "ptx.cuh"
 
 namespace b200a {
@@ -46,38 +45,26 @@ constexpr int kRsMaxTiles = 128;     // groups of 8 phases  (new' <= 1024)
 constexpr int kRsSmemBudget = 224 * 1024;
 
 struct RsTile {  // one group of 8 phases
-  int kstart;      // first tap of its first k-step (multiple of 8)
-  int nsteps;      // 8-tap k-steps covering the union of the group's live taps
-  int frag_off;    // first step in the TF32 fragment array
-  int frag16_off;  // first 16-tap step in the bf16 fragment array
+  int kstart;    // first tap of its first k-step (multiple of 8)
+  int nsteps;    // 8-tap k-steps covering the union of the group's live taps
+  int frag_off;  // first step in the TF32 fragment array
+  int pad;
 };
+static_assert(sizeof(RsTile) == 16, "the mma kernel's shared-memory layout assumes 16-byte tiles");
 
 struct RsHeader {
   uint32_t magic;
   int32_t orig_r, new_r, width, taps, max_support, n_tiles, total_steps;
-  int32_t simt_tap_floats;  // size of the SIMT tap table (floats)
-  int32_t total_steps16;    // 16-tap steps over all groups (bf16 fragments)
-  int32_t r3_ok;            // 1: every group of 4 phases spans at most kR3Len taps (resample_r3_kernel applies)
-  int32_t tc_ok;            // 1: the banded tcgen05 plan fits (resample_tc_kernel applies)
-  int32_t reserved[4];
+  int32_t tc_ok;  // 1: the banded tcgen05 plan fits (resample_tc_kernel applies)
+  int32_t reserved[7];
 };
 static_assert(sizeof(RsHeader) == 64, "header is 64 bytes");
 
 struct RsLayout {
-  size_t header, support, tiles, frags, frags16, sgroups, staps, r3base, r3taps, tcplan, tcblocks, total;
+  size_t header, support, tiles, frags, tcblocks, total;
 };
 
 constexpr int kTcBBudgetBytes = 64 * 1024;  // banded tap blocks of the tcgen05 kernel
-constexpr int kR3Len = 44;      // taps per phase quad held in registers (34 live + 3 x 2.76 drift at 441:160, padded)
-constexpr int kR3Warps = 8;     // warps per CTA == phase quads per CTA (a multiple of 4: registers are granted per 4 warps)
-constexpr int kR3MaxCluster = 8;
-
-struct RsSimtGroup {  // one group of 8 phases for the SIMT kernel
-  int base;  // first tap (xp-relative) any phase of the group uses
-  int len;   // taps visited (multiple of 8; zero padded)
-  int off;   // float offset of the group's [len][8] tap block in the tap table
-  int pad;
-};
 
 inline int rs_tiles(int new_r) { return (new_r + 7) / 8; }
 
@@ -93,20 +80,7 @@ inline RsLayout rs_layout(int new_r, int taps) {
   l.frags = off;  // worst case: every group spans every tap
   const size_t nt = rs_tiles(new_r) <= kRsMaxTiles ? rs_tiles(new_r) : 0;
   off = align_up(off + sizeof(float4) * 32 * nt * ((size_t)taps / 8 + 2), 256);
-  l.frags16 = off;  // bf16 hi / lo fragments of the 16-tap steps (resample_mma_kernel<true>)
-  off = align_up(off + sizeof(uint4) * 32 * nt * ((size_t)taps / 16 + 2), 256);
-  l.sgroups = off;
-  off = align_up(off + sizeof(RsSimtGroup) * (size_t)rs_tiles(new_r), 256);
-  l.staps = off;  // worst case: every group spans every tap
-  off = align_up(off + sizeof(float) * 8 * (size_t)rs_tiles(new_r) * ((size_t)taps + 8), 256);
-  const size_t quads = ((size_t)new_r + 3) / 4;
-  l.r3base = off;
-  off = align_up(off + sizeof(int) * quads, 256);
-  l.r3taps = off;
-  off = align_up(off + sizeof(float4) * kR3Len * quads, 256);
-  l.tcplan = off;  // (spare) + the banded bf16 tap blocks of resample_tc_kernel
-  off = align_up(off + 1024, 256);
-  l.tcblocks = off;
+  l.tcblocks = off;  // the banded bf16 tap blocks of resample_tc_kernel
   off = align_up(off + (size_t)kTcBBudgetBytes, 256);
   l.total = off;
   return l;
@@ -148,8 +122,6 @@ __global__ void resample_support_kernel(const float* __restrict__ kernel, int ne
   }
 }
 
-// Per group of 8 phases: the k-steps its live taps span, and the taps split into TF32 hi/lo parts in
-// mma.m16n8k8 B-fragment order (B[k][n] = K[8 t + n][kstart + k]).
 // (x, y) -> packed bf16 pair (x in the low half) and the packed pair of the residuals
 __device__ __forceinline__ void rs_split_bf16x2(float x, float y, uint32_t& hi, uint32_t& lo) {
   asm("cvt.rn.bf16x2.f32 %0, %1, %2;" : "=r"(hi) : "f"(y), "f"(x));
@@ -157,28 +129,28 @@ __device__ __forceinline__ void rs_split_bf16x2(float x, float y, uint32_t& hi, 
   asm("cvt.rn.bf16x2.f32 %0, %1, %2;" : "=r"(lo) : "f"(ry), "f"(rx));
 }
 
+// Per group of 8 phases: the k-steps its live taps span, and the taps split into TF32 hi/lo parts in
+// mma.m16n8k8 B-fragment order (B[k][n] = K[8 t + n][kstart + k]).
 __global__ void resample_plan_kernel(const float* __restrict__ kernel, const int2* __restrict__ support, int new_r,
-                                     int taps, int n_tiles, RsHeader* hdr, RsTile* tiles, float4* frags, uint4* frags16) {
+                                     int taps, int n_tiles, RsHeader* hdr, RsTile* tiles, float4* frags) {
   if (threadIdx.x == 0) {
-    int acc = 0, acc16 = 0;
+    int acc = 0;
     for (int t = 0; t < n_tiles; ++t) {
       int lo = taps, hi = 0;
       for (int j = 8 * t; j < min(8 * t + 8, new_r); ++j) {
         const int2 sp = support[j];
         if (sp.y > 0) { lo = min(lo, sp.x); hi = max(hi, sp.x + sp.y); }
       }
-      RsTile rt{0, 0, acc, acc16};
+      RsTile rt{0, 0, acc, 0};
       if (hi > lo) {
         rt.kstart = lo & ~7;
         rt.nsteps = (hi - rt.kstart + 7) / 8;
       }
       tiles[t] = rt;
       acc += rt.nsteps;
-      acc16 += (rt.nsteps + 1) / 2;
     }
     hdr->n_tiles = n_tiles;
     hdr->total_steps = acc;
-    hdr->total_steps16 = acc16;
   }
   __syncthreads();
   for (int t = 0; t < n_tiles; ++t) {
@@ -193,24 +165,6 @@ __global__ void resample_plan_kernel(const float* __restrict__ kernel, const int
       const float b1h = __uint_as_float(__float_as_uint(b1) & 0xffffe000u);
       frags[(size_t)(rt.frag_off + s) * 32 + lane] = make_float4(b0h, b1h, b0 - b0h, b1 - b1h);
     }
-    // 16-tap steps for mma.m16n8k16 bf16: the instruction's k index is a PERMUTATION of the taps chosen so that a
-    // thread's A elements (k = 2c, 2c+1, 2c+8, 2c+9) are taps c, c+4, c+8, c+12 of the step -- the same
-    // conflict-free shared-memory reads as the 8-tap TF32 steps.  B[k][n] follows the same permutation.
-    const int n16 = (rt.nsteps + 1) / 2;
-    for (int i = threadIdx.x; i < n16 * 32; i += blockDim.x) {
-      const int s = i >> 5, lane = i & 31;
-      const int j = 8 * t + (lane >> 2), c = lane & 3;
-      float v[4];
-#pragma unroll
-      for (int q = 0; q < 4; ++q) {
-        const int k = rt.kstart + 16 * s + c + 4 * q;
-        v[q] = (j < new_r && k < taps && k < rt.kstart + 8 * rt.nsteps) ? kernel[(size_t)j * taps + k] : 0.f;
-      }
-      uint4 f;
-      rs_split_bf16x2(v[0], v[1], f.x, f.z);  // b0: taps c, c + 4
-      rs_split_bf16x2(v[2], v[3], f.y, f.w);  // b1: taps c + 8, c + 12
-      frags16[(size_t)(rt.frag16_off + s) * 32 + lane] = f;
-    }
   }
 }
 
@@ -222,7 +176,6 @@ struct RsParams {
   const RsHeader* hdr;
   const RsTile* tiles;
   const float4* frags;
-  const uint4* frags16;
   int orig_r, new_r, width, taps, n_tiles;
   int64_t frames;           // output frames per row = ceil(out_len / new_r)
   int64_t blocks_per_row;   // ceil(frames / kRsFrames)
@@ -230,7 +183,7 @@ struct RsParams {
   int xs_floats;            // floats per staging buffer
   int frag_smem_bytes;      // shared memory granted to the fragment copy (0: read them from global)
   int row_spread;           // 1, 2 or 4: frame distance of the 8 rows one A-fragment load touches
-  int skip_if_r3_ok;        // launched behind resample_r3_kernel (1) / resample_tc_kernel (2): leave when the header says that kernel did the work
+  int behind_tc;            // launched behind resample_tc_kernel: leave when the header says that kernel did the work
   int out_pair;             // new' and the row pitch are even and `out` is 8-byte aligned: phase pairs are one float2 store
 };
 
@@ -287,16 +240,7 @@ __device__ __forceinline__ int frame_of(int spread, int h, int rho) {
   return 16 * h + rho;
 }
 
-__device__ __forceinline__ void mma_bf16_16816(float (&d)[4], const uint32_t (&a)[4], uint32_t b0, uint32_t b1) {
-  asm volatile(
-      "mma.sync.aligned.m16n8k16.row.col.f32.bf16.bf16.f32 {%0,%1,%2,%3}, {%4,%5,%6,%7}, {%8,%9}, {%0,%1,%2,%3};"
-      : "+f"(d[0]), "+f"(d[1]), "+f"(d[2]), "+f"(d[3])
-      : "r"(a[0]), "r"(a[1]), "r"(a[2]), "r"(a[3]), "r"(b0), "r"(b1));
-}
-
-// BF16 == false: m16n8k8 TF32 x 3 (2^-21 relative);  BF16 == true: m16n8k16 bf16 x 3 (2^-16 relative, half the
-// tensor-pipe time: the TF32 variant is throttled by the math pipe, profiles/r1_resample_v4.txt)
-template <bool BF16>
+// m16n8k8 TF32 x 3 (2^-21 relative)
 __global__ void __launch_bounds__(kRsMaxWarps * 32, 1) resample_mma_kernel(const RsParams p) {
   extern __shared__ __align__(128) unsigned char smem_raw[];
   float* s_x = reinterpret_cast<float*>(smem_raw);                              // [2][xs_floats]
@@ -305,14 +249,12 @@ __global__ void __launch_bounds__(kRsMaxWarps * 32, 1) resample_mma_kernel(const
   float4* s_frags = reinterpret_cast<float4*>(s_tiles + ((p.n_tiles + 3) & ~3));  // optional
 
   const int tid = threadIdx.x, lane = tid & 31, warp = tid >> 5;
-  if ((p.skip_if_r3_ok == 1 && p.hdr->r3_ok != 0) || (p.skip_if_r3_ok == 2 && p.hdr->tc_ok != 0)) return;
+  if (p.behind_tc && p.hdr->tc_ok != 0) return;
   for (int i = tid; i < p.n_tiles; i += blockDim.x) s_tiles[i] = p.tiles[i];
-  const int total_steps = BF16 ? p.hdr->total_steps16 : p.hdr->total_steps;
+  const int total_steps = p.hdr->total_steps;
   const bool frags_in_smem = (size_t)total_steps * 512 <= (size_t)p.frag_smem_bytes;
-  if (frags_in_smem) {
-    const float4* src = BF16 ? reinterpret_cast<const float4*>(p.frags16) : p.frags;
-    for (int i = tid; i < total_steps * 32; i += blockDim.x) s_frags[i] = src[i];
-  }
+  if (frags_in_smem)
+    for (int i = tid; i < total_steps * 32; i += blockDim.x) s_frags[i] = p.frags[i];
   if (tid == 0) {
     mbar_init(s_bar + 0, 1);
     mbar_init(s_bar + 1, 1);
@@ -367,31 +309,6 @@ __global__ void __launch_bounds__(kRsMaxWarps * 32, 1) resample_mma_kernel(const
 #pragma unroll
           for (int q = 0; q < 4; ++q) d[h][ch][q] = 0.f;
       auto contract = [&](auto in_smem) {
-        if constexpr (BF16) {
-          const uint4* frg = (decltype(in_smem)::value ? reinterpret_cast<const uint4*>(s_frags) : p.frags16) +
-                             (size_t)rt.frag16_off * 32 + lane;
-          const int n16 = (rt.nsteps + 1) >> 1;
-#pragma unroll 2
-          for (int s = 0; s < n16; ++s) {
-            uint4 bf;
-            if constexpr (decltype(in_smem)::value) bf = frg[(size_t)s * 32];
-            else bf = __ldg(frg + (size_t)s * 32);
-#pragma unroll
-            for (int h = 0; h < 2; ++h) {
-              // k = 2c, 2c+1 <-> taps c, c+4;  k = 2c+8, 2c+9 <-> taps c+8, c+12 (see resample_plan_kernel)
-              const float* lo_row = arow[2 * h] + 16 * s;
-              const float* hi_row = arow[2 * h + 1] + 16 * s;
-              uint32_t ah[4], al[4];
-              rs_split_bf16x2(lo_row[0], lo_row[4], ah[0], al[0]);
-              rs_split_bf16x2(hi_row[0], hi_row[4], ah[1], al[1]);
-              rs_split_bf16x2(lo_row[8], lo_row[12], ah[2], al[2]);
-              rs_split_bf16x2(hi_row[8], hi_row[12], ah[3], al[3]);
-              mma_bf16_16816(d[h][0], ah, bf.x, bf.y);
-              mma_bf16_16816(d[h][1], al, bf.x, bf.y);
-              mma_bf16_16816(d[h][2], ah, bf.z, bf.w);
-            }
-          }
-        } else {
         const float4* frg = (decltype(in_smem)::value ? s_frags : p.frags) + (size_t)rt.frag_off * 32 + lane;
 #pragma unroll 2
         for (int s = 0; s < rt.nsteps; ++s) {
@@ -409,7 +326,6 @@ __global__ void __launch_bounds__(kRsMaxWarps * 32, 1) resample_mma_kernel(const
             mma_tf32(d[h][1], lo, __float_as_uint(bf.x), __float_as_uint(bf.y));
             mma_tf32(d[h][2], hi, __float_as_uint(bf.z), __float_as_uint(bf.w));
           }
-        }
         }
       };
       if (frags_in_smem) contract(std::true_type{});
@@ -434,475 +350,6 @@ __global__ void __launch_bounds__(kRsMaxWarps * 32, 1) resample_mma_kernel(const
     }
     __syncthreads();  // everyone is done with buffer b before it is refilled
   }
-}
-
-// ---- SIMT kernel tables: per group of 8 phases the union of their live taps, zero padded to a multiple of 8,
-// stored tap-major ([i][8 phases]) so one step's taps are one 32-byte broadcast read.
-__global__ void resample_simt_plan_kernel(const float* __restrict__ kernel, const int2* __restrict__ support, int new_r,
-                                          int taps, int n_groups, RsHeader* hdr, RsSimtGroup* groups, float* table) {
-  if (threadIdx.x == 0) {
-    int acc = 0;
-    for (int g = 0; g < n_groups; ++g) {
-      int lo = taps, hi = 0;
-      for (int j = 8 * g; j < min(8 * g + 8, new_r); ++j) {
-        const int2 sp = support[j];
-        if (sp.y > 0) { lo = min(lo, sp.x); hi = max(hi, sp.x + sp.y); }
-      }
-      RsSimtGroup sg{0, 0, acc, 0};
-      if (hi > lo) {
-        sg.base = lo;
-        sg.len = (hi - lo + 7) & ~7;
-      }
-      groups[g] = sg;
-      acc += sg.len * 8;
-    }
-    hdr->simt_tap_floats = acc;
-  }
-  __syncthreads();
-  for (int g = 0; g < n_groups; ++g) {
-    const RsSimtGroup sg = groups[g];
-    for (int e = threadIdx.x; e < sg.len * 8; e += blockDim.x) {
-      const int i = e >> 3, q = e & 7, j = 8 * g + q, t = sg.base + i;
-      float v = 0.f;
-      if (j < new_r && t < taps) {
-        const int2 sp = support[j];
-        if (t >= sp.x && t < sp.x + sp.y) v = kernel[(size_t)j * taps + t];
-      }
-      table[sg.off + e] = v;
-    }
-  }
-}
-
-struct RsSimtParams {
-  const float* wave;
-  int64_t rows, length, row_stride;
-  float* out;
-  int64_t out_row_stride, out_len;
-  const RsHeader* hdr;
-  const RsSimtGroup* groups;
-  const float* table;
-  int orig_r, new_r, width, n_groups;
-  int tap_floats;        // shared memory granted to the tap table (floats)
-  int64_t frames;        // output frames per row
-  int64_t halves;        // 32-frame half-chunks per row
-  int64_t total_halves;  // rows * halves
-  int slot_floats;       // floats per ring slot
-  int out_vec;           // 1: every frame's 8-phase run may be stored as two float4
-};
-
-constexpr int kSimtMaxWarps = 12;
-
-// Stage the samples of half-chunk (row, hk) into a ring slot: xs[q] = xp[32 hk orig' + q - shift] with
-// xp[m] = x[m - width] (zero outside the signal).  Same alignment rule as rs_fill.
-__device__ __forceinline__ int simt_fill(const RsSimtParams& p, int64_t row, int64_t hk, float* xs, uint64_t* bar,
-                                         int tid, int nthreads) {
-  const int64_t T0 = hk * 32 * p.orig_r - p.width;
-  const float* x = p.wave + row * p.row_stride;
-  const int a0 = (int)((reinterpret_cast<uintptr_t>(x) >> 2) & 3);
-  const int shift = (int)((((a0 + T0) % 4) + 4) % 4);
-  const int64_t span = (int64_t)32 * p.orig_r + 2 * p.width;
-  const int64_t lo = T0 < 0 ? 0 : T0;
-  int64_t hi = T0 + span;
-  if (hi > p.length) hi = p.length;
-  if (hi < lo) hi = lo;
-  const int64_t lo_a = lo + ((4 - ((a0 + lo) & 3)) & 3);
-  const int64_t hi_a = hi - ((a0 + hi) & 3);
-  const int q_lo = (int)(lo - T0) + shift, q_hi = (int)(hi - T0) + shift;
-  if (q_lo > 0 && T0 < 0)
-    for (int q = tid; q < q_lo; q += nthreads) xs[q] = 0.f;
-  if (hi < T0 + span)
-    for (int q = q_hi + tid; q < p.slot_floats; q += nthreads) xs[q] = 0.f;
-  if (hi_a > lo_a) {
-    const int head = (int)(lo_a - lo), tail = (int)(hi - hi_a);
-    if (tid < head) xs[q_lo + tid] = x[lo + tid];
-    else if (tid >= 32 && tid < 32 + tail) xs[(int)(hi_a - T0) + shift + (tid - 32)] = x[hi_a + (tid - 32)];
-  } else {
-    for (int q = q_lo + tid; q < q_hi; q += nthreads) xs[q] = x[T0 + q - shift];
-  }
-  if (tid == 0) {
-    if (hi_a > lo_a) {
-      const uint32_t bytes = (uint32_t)(hi_a - lo_a) * 4u;
-      mbar_expect_tx(bar, bytes);
-      bulk_g2s(xs + (lo_a - T0) + shift, x + lo_a, bytes, bar);
-    } else {
-      mbar_arrive(bar);
-    }
-  }
-  return shift;
-}
-// where sample xp[32 hk orig'] of half-chunk (row, hk) sits in its slot (simt_fill's `shift`)
-__device__ __forceinline__ int simt_shift(const RsSimtParams& p, int64_t row, int64_t hk) {
-  const int64_t T0 = hk * 32 * p.orig_r - p.width;
-  const int a0 = (int)((reinterpret_cast<uintptr_t>(p.wave + row * p.row_stride) >> 2) & 3);
-  return (int)((((a0 + T0) % 4) + 4) % 4);
-}
-
-__global__ void __launch_bounds__(kSimtMaxWarps * 32, 1) resample_simt_kernel(const RsSimtParams p) {
-  extern __shared__ __align__(128) unsigned char smem_raw[];
-  float* s_x = reinterpret_cast<float*>(smem_raw);                                   // [3][slot_floats]
-  float* s_taps = s_x + 3 * (size_t)p.slot_floats;                                   // [tap_floats]
-  RsSimtGroup* s_groups = reinterpret_cast<RsSimtGroup*>(s_taps + ((p.tap_floats + 3) & ~3));  // [n_groups]
-  uint64_t* s_bar = reinterpret_cast<uint64_t*>(s_groups + p.n_groups);              // [3]
-
-  const int tid = threadIdx.x, lane = tid & 31, warp = tid >> 5, n_warps = blockDim.x >> 5;
-  const int tap_need = p.hdr->simt_tap_floats;
-  const bool taps_in_smem = tap_need <= p.tap_floats;
-  if (taps_in_smem)
-    for (int i = tid; i < tap_need; i += blockDim.x) s_taps[i] = p.table[i];
-  for (int i = tid; i < p.n_groups; i += blockDim.x) s_groups[i] = p.groups[i];
-  if (tid < 3) mbar_init(s_bar + tid, 1);
-  asm volatile("fence.mbarrier_init.release.cluster;" ::: "memory");
-  __syncthreads();
-
-  // this CTA's contiguous run of half-chunks [h0, h1) in (row, half) order
-  const int64_t h0 = p.total_halves * blockIdx.x / gridDim.x, h1 = p.total_halves * (blockIdx.x + 1) / gridDim.x;
-  if (h0 >= h1) return;
-  uint32_t phase_bits = 0;  // bit i: parity the next wait on slot i expects
-  {
-    const int64_t row = h0 / p.halves;
-    simt_fill(p, row, h0 - row * p.halves, s_x + (size_t)(h0 % 3) * p.slot_floats, s_bar + (h0 % 3), tid, blockDim.x);
-  }
-  __syncthreads();
-  const bool vec_ok = p.out_vec != 0;
-  for (int64_t s = h0; s <= h1; ++s) {
-    const int slot_hi = (int)(s % 3), slot_lo = (int)((s + 2) % 3), slot_nx = (int)((s + 1) % 3);
-    if (s + 1 < h1) {  // the slot of half-chunk s - 2: its last readers left at the barrier that ended step s - 1
-      const int64_t nrow = (s + 1) / p.halves;
-      asm volatile("fence.proxy.async.shared::cta;" ::: "memory");
-      simt_fill(p, nrow, (s + 1) - nrow * p.halves, s_x + (size_t)slot_nx * p.slot_floats, s_bar + slot_nx, tid,
-                blockDim.x);
-    }
-    const bool has_hi = s < h1, has_lo = s > h0;
-    if (has_hi) {
-      mbar_wait(s_bar + slot_hi, (phase_bits >> slot_hi) & 1u);
-      phase_bits ^= 1u << slot_hi;
-    }
-    // frames of this thread: lane of the older half-chunk (s - 1) and lane of the newer one (s)
-    const int64_t hb = has_hi ? s : s - 1, ha = has_lo ? s - 1 : s;  // an absent side mirrors the present one
-    const int64_t row_a = ha / p.halves, row_b = hb / p.halves;
-    const int64_t fa = (ha - row_a * p.halves) * 32 + lane, fb = (hb - row_b * p.halves) * 32 + lane;
-    const float* xa = s_x + (size_t)(has_lo ? slot_lo : slot_hi) * p.slot_floats +
-                      simt_shift(p, row_a, ha - row_a * p.halves) + lane * p.orig_r;
-    const float* xb = s_x + (size_t)(has_hi ? slot_hi : slot_lo) * p.slot_floats +
-                      simt_shift(p, row_b, hb - row_b * p.halves) + lane * p.orig_r;
-    const bool st_a = has_lo && fa < p.frames, st_b = has_hi && fb < p.frames;
-    float* oa = p.out + row_a * p.out_row_stride + fa * p.new_r;
-    float* ob = p.out + row_b * p.out_row_stride + fb * p.new_r;
-    const int64_t na = fa * p.new_r, nb = fb * p.new_r;  // output index of phase 0 of the two frames
-    for (int g = 2 * warp + (int)(s & 1); g < p.n_groups; g += 2 * n_warps) {
-      const RsSimtGroup sg = s_groups[g];
-      const float* ta = xa + sg.base;
-      const float* tb = xb + sg.base;
-      uint64_t acc[8];
-#pragma unroll
-      for (int q = 0; q < 8; ++q) acc[q] = 0ull;
-      auto fir = [&](auto in_smem) {
-        const float4* tp = reinterpret_cast<const float4*>((decltype(in_smem)::value ? s_taps : p.table) + sg.off);
-        // software pipelined over blocks of 4 taps: the loads of block k + 1 are in flight while block k is multiplied
-        float4 tq[2][8];
-        float va[2][4], vb[2][4];
-        auto load = [&](auto bi, int i4) {
-          constexpr int B = decltype(bi)::value;
-#pragma unroll
-          for (int u = 0; u < 4; ++u) {
-            va[B][u] = ta[i4 + u];
-            vb[B][u] = tb[i4 + u];
-            if constexpr (decltype(in_smem)::value) {
-              tq[B][2 * u] = tp[2 * (i4 + u)];
-              tq[B][2 * u + 1] = tp[2 * (i4 + u) + 1];
-            } else {
-              tq[B][2 * u] = __ldg(tp + 2 * (i4 + u));
-              tq[B][2 * u + 1] = __ldg(tp + 2 * (i4 + u) + 1);
-            }
-          }
-        };
-        auto mac = [&](auto bi) {
-          constexpr int B = decltype(bi)::value;
-#pragma unroll
-          for (int u = 0; u < 4; ++u) {
-            const uint64_t xx = pk2(va[B][u], vb[B][u]);
-            const float4 t0 = tq[B][2 * u], t1 = tq[B][2 * u + 1];
-            acc[0] = fma2_raw(xx, pk2(t0.x, t0.x), acc[0]);
-            acc[1] = fma2_raw(xx, pk2(t0.y, t0.y), acc[1]);
-            acc[2] = fma2_raw(xx, pk2(t0.z, t0.z), acc[2]);
-            acc[3] = fma2_raw(xx, pk2(t0.w, t0.w), acc[3]);
-            acc[4] = fma2_raw(xx, pk2(t1.x, t1.x), acc[4]);
-            acc[5] = fma2_raw(xx, pk2(t1.y, t1.y), acc[5]);
-            acc[6] = fma2_raw(xx, pk2(t1.z, t1.z), acc[6]);
-            acc[7] = fma2_raw(xx, pk2(t1.w, t1.w), acc[7]);
-          }
-        };
-        using B0 = std::integral_constant<int, 0>;
-        using B1 = std::integral_constant<int, 1>;
-        if (sg.len > 0) load(B0{}, 0);
-#pragma unroll 1
-        for (int i8 = 0; i8 < sg.len; i8 += 8) {  // len is a multiple of 8
-          load(B1{}, i8 + 4);
-          mac(B0{});
-          if (i8 + 8 < sg.len) load(B0{}, i8 + 8);
-          mac(B1{});
-        }
-      };
-      if (taps_in_smem) fir(std::true_type{});
-      else fir(std::false_type{});
-      float ya[8], yb[8];
-#pragma unroll
-      for (int q = 0; q < 8; ++q) {
-        const float2 v = upk2(acc[q]);
-        ya[q] = v.x;
-        yb[q] = v.y;
-      }
-      const int j0 = 8 * g;
-      const bool full = j0 + 8 <= p.new_r && vec_ok;
-      auto store = [&](float* o, int64_t n0, const float (&y)[8]) {
-        if (full && n0 + j0 + 8 <= p.out_len) {
-          *reinterpret_cast<float4*>(o + j0) = make_float4(y[0], y[1], y[2], y[3]);
-          *reinterpret_cast<float4*>(o + j0 + 4) = make_float4(y[4], y[5], y[6], y[7]);
-        } else {
-#pragma unroll
-          for (int q = 0; q < 8; ++q)
-            if (j0 + q < p.new_r && n0 + j0 + q < p.out_len) o[j0 + q] = y[q];
-        }
-      };
-      if (st_a) store(oa, na, ya);
-      if (st_b) store(ob, nb, yb);
-    }
-    __syncthreads();  // every reader of slot_lo is done: the next step's copy may overwrite it
-  }
-}
-
-// ---- cluster kernel tables: per QUAD of 4 phases the first live tap and kR3Len taps x 4 phases (zero padded) -------
-__global__ void resample_r3_plan_kernel(const float* __restrict__ kernel, const int2* __restrict__ support, int new_r,
-                                        int taps, int n_quads, RsHeader* hdr, int* qbase, float4* qtaps) {
-  __shared__ int s_ok;
-  if (threadIdx.x == 0) s_ok = 1;
-  __syncthreads();
-  for (int q = threadIdx.x; q < n_quads; q += blockDim.x) {
-    int lo = taps, hi = 0;
-    for (int j = 4 * q; j < min(4 * q + 4, new_r); ++j) {
-      const int2 sp = support[j];
-      if (sp.y > 0) { lo = min(lo, sp.x); hi = max(hi, sp.x + sp.y); }
-    }
-    if (hi <= lo) lo = hi = 0;
-    if (hi - lo > kR3Len) s_ok = 0;
-    qbase[q] = lo;
-  }
-  __syncthreads();
-  for (int e = threadIdx.x; e < n_quads * kR3Len; e += blockDim.x) {
-    const int q = e / kR3Len, i = e - q * kR3Len, t = qbase[q] + i;
-    float v[4] = {0.f, 0.f, 0.f, 0.f};
-#pragma unroll
-    for (int r = 0; r < 4; ++r) {
-      const int j = 4 * q + r;
-      if (j < new_r && t < taps) {
-        const int2 sp = support[j];
-        if (t >= sp.x && t < sp.x + sp.y) v[r] = kernel[(size_t)j * taps + t];
-      }
-    }
-    qtaps[e] = make_float4(v[0], v[1], v[2], v[3]);
-  }
-  if (threadIdx.x == 0) hdr->r3_ok = s_ok;
-}
-
-// ================================================================================================
-// Cluster kernel (resample_r3_kernel): the taps never leave the register file.
-//   A register-tiled FIR is bound by shared-memory wavefronts unless BOTH operands of an FMA are reused from
-//   registers (docs/KERNEL_NOTES.md).  Here a warp owns ONE quad of 4 output phases for the whole kernel and keeps
-//   its 4 x kR3Len taps in 176 registers; lanes are the 32 frames of a tile, so the only shared-memory traffic is one
-//   conflict-free 4-byte read per tap position, feeding two FFMA2 (4 phases) with the sample as the broadcast operand.
-//   160 phases = 40 quads need 40 such warps; at ~200 registers per thread an SM holds 8 (registers are granted per 4
-//   warps: 10 x 200 does not fit), so a CLUSTER of 5 CTAs covers the phases and shares every staged tile: each CTA
-//   fetches a fifth of the tile's samples with ONE bulk copy that is MULTICAST into the same offset of all the CTAs'
-//   shared memory (every HBM byte is read once), through a 3-slot ring
-//   with cluster-scope full / empty mbarriers.
-// ================================================================================================
-struct R3Params {
-  const float* wave;
-  int64_t rows, length, row_stride;
-  float* out;
-  int64_t out_row_stride, out_len;
-  const RsHeader* hdr;
-  const int* qbase;
-  const float4* qtaps;
-  int orig_r, new_r, width, n_quads, csize;
-  int64_t frames, tiles_per_row, total_tiles;
-  int slot_floats, out_vec;
-};
-
-__device__ __forceinline__ uint32_t cluster_ctarank() {
-  uint32_t r;
-  asm volatile("mov.u32 %0, %%cluster_ctarank;" : "=r"(r));
-  return r;
-}
-__device__ __forceinline__ void cluster_sync_all() {
-  asm volatile("barrier.cluster.arrive.release.aligned;" ::: "memory");
-  asm volatile("barrier.cluster.wait.acquire.aligned;" ::: "memory");
-}
-// arrive on the mbarrier at the same shared-memory offset in CTA `rank` of the cluster
-__device__ __forceinline__ void mbar_arrive_remote(uint64_t* bar, uint32_t rank) {
-  uint32_t raddr;
-  asm volatile("mapa.shared::cluster.u32 %0, %1, %2;" : "=r"(raddr) : "r"(smem_u32(bar)), "r"(rank));
-  asm volatile("mbarrier.arrive.release.cluster.shared::cluster.b64 _, [%0];" ::"r"(raddr) : "memory");
-}
-// bulk copy global -> the same shared-memory offset of every CTA in `mask`, completing bytes on each one's mbarrier
-__device__ __forceinline__ void bulk_g2s_multicast(void* dst, const void* src, uint32_t bytes, uint64_t* bar, uint16_t mask) {
-  asm volatile(
-      "cp.async.bulk.shared::cluster.global.mbarrier::complete_tx::bytes.multicast::cluster [%0], [%1], %2, [%3], %4;" ::"r"(
-          smem_u32(dst)),
-      "l"(src), "r"(bytes), "r"(smem_u32(bar)), "h"(mask)
-      : "memory");
-}
-__device__ __forceinline__ void mbar_wait_cluster(uint64_t* bar, uint32_t parity) {
-  const uint32_t addr = smem_u32(bar);
-  for (int spin = 0; spin < (1 << 22); ++spin) {
-    uint32_t ok;
-    asm volatile(
-        "{\n.reg .pred p;\n"
-        "mbarrier.try_wait.parity.acquire.cluster.shared::cta.b64 p, [%1], %2, %3;\n"
-        "selp.u32 %0, 1, 0, p;\n}"
-        : "=r"(ok)
-        : "r"(addr), "r"(parity), "r"(2000u)
-        : "memory");
-    if (ok) return;
-  }
-  __trap();
-}
-
-// Stage tile (row, f0) into ring slot `xs` of EVERY CTA of the cluster: local zero fill / unaligned head and tail by all
-// threads of each CTA, and this CTA's share of the 16-byte aligned body as one multicast bulk copy.  Returns `shift`.
-__device__ __forceinline__ void r3_fill(const R3Params& p, int64_t row, int64_t f0, float* xs, uint64_t* full, uint32_t crank,
-                                        int tid, int nthreads) {
-  const int64_t T0 = f0 * p.orig_r - p.width;
-  const float* x = p.wave + row * p.row_stride;
-  const int a0 = (int)((reinterpret_cast<uintptr_t>(x) >> 2) & 3);
-  const int shift = (int)((((a0 + T0) % 4) + 4) % 4);
-  const int64_t span = (int64_t)32 * p.orig_r + 2 * p.width + 16;  // + the zero-tap tail of a padded quad
-  const int64_t lo = T0 < 0 ? 0 : T0;
-  int64_t hi = T0 + span;
-  if (hi > p.length) hi = p.length;
-  if (hi < lo) hi = lo;
-  const int64_t lo_a = lo + ((4 - ((a0 + lo) & 3)) & 3);
-  const int64_t hi_a = hi - ((a0 + hi) & 3);
-  const int q_lo = (int)(lo - T0) + shift, q_hi = (int)(hi - T0) + shift;
-  if (q_lo > 0 && T0 < 0)
-    for (int q = tid; q < q_lo; q += nthreads) xs[q] = 0.f;
-  if (hi < T0 + span)
-    for (int q = q_hi + tid; q < p.slot_floats; q += nthreads) xs[q] = 0.f;
-  if (hi_a > lo_a) {
-    const int head = (int)(lo_a - lo), tail = (int)(hi - hi_a);
-    if (tid < head) xs[q_lo + tid] = x[lo + tid];
-    else if (tid >= 32 && tid < 32 + tail) xs[(int)(hi_a - T0) + shift + (tid - 32)] = x[hi_a + (tid - 32)];
-  } else {
-    for (int q = q_lo + tid; q < q_hi; q += nthreads) xs[q] = x[T0 + q - shift];
-  }
-  if (tid == 0) {
-    if (hi_a > lo_a) {
-      const int64_t n_al = hi_a - lo_a;                                   // multiple of 4 floats
-      const int64_t chunk = ((n_al / 4 + p.csize - 1) / p.csize) * 4;     // floats per CTA, multiple of 4
-      mbar_expect_tx(full, (uint32_t)n_al * 4u);                          // the whole body lands in every CTA
-      const int64_t c0 = lo_a + (int64_t)crank * chunk;
-      int64_t c1 = c0 + chunk;
-      if (c1 > hi_a) c1 = hi_a;
-      if (c1 > c0)
-        bulk_g2s_multicast(xs + (c0 - T0) + shift, x + c0, (uint32_t)(c1 - c0) * 4u, full, (uint16_t)((1u << p.csize) - 1u));
-    } else {
-      mbar_arrive(full);
-    }
-  }
-}
-__device__ __forceinline__ int r3_shift(const R3Params& p, int64_t row, int64_t f0) {
-  const int64_t T0 = f0 * p.orig_r - p.width;
-  const int a0 = (int)((reinterpret_cast<uintptr_t>(p.wave + row * p.row_stride) >> 2) & 3);
-  return (int)((((a0 + T0) % 4) + 4) % 4);
-}
-
-__global__ void __maxnreg__(224) resample_r3_kernel(const R3Params p, int require_flag) {
-  extern __shared__ __align__(128) unsigned char smem_raw[];
-  float* s_x = reinterpret_cast<float*>(smem_raw);                                   // [3][slot_floats]
-  uint64_t* s_full = reinterpret_cast<uint64_t*>(s_x + 3 * (size_t)p.slot_floats);   // [3]
-  uint64_t* s_empty = s_full + 3;                                                    // [3]
-  if (require_flag && p.hdr->r3_ok == 0) return;  // (uniform over the grid) the mma kernel launched next does the work
-
-  const int tid = threadIdx.x, lane = tid & 31, warp = tid >> 5;
-  const uint32_t crank = cluster_ctarank();
-  const int64_t cid = blockIdx.x / p.csize, n_clusters = gridDim.x / p.csize;
-  if (tid < 3) {
-    mbar_init(s_full + tid, 1);
-    mbar_init(s_empty + tid, p.csize);
-  }
-  asm volatile("fence.mbarrier_init.release.cluster;" ::: "memory");
-  cluster_sync_all();  // every CTA's barriers exist before anyone multicasts into it or arrives on it
-
-  // this warp's quad of phases and its taps (registers for the rest of the kernel)
-  const int quad = (int)crank * kR3Warps + warp;
-  const bool active = quad < p.n_quads;
-  float4 tp[kR3Len];
-  int qb = 0;
-  if (active) {
-    qb = p.qbase[quad];
-#pragma unroll
-    for (int i = 0; i < kR3Len; ++i) tp[i] = __ldg(p.qtaps + (size_t)quad * kR3Len + i);
-  } else {
-#pragma unroll
-    for (int i = 0; i < kR3Len; ++i) tp[i] = make_float4(0.f, 0.f, 0.f, 0.f);
-  }
-  const int j0 = 4 * quad;
-
-  // tiles of this cluster: T(n) = cid + n * n_clusters
-  auto tile_of = [&](int64_t n, int64_t& row, int64_t& f0) {
-    const int64_t t = cid + n * n_clusters;
-    row = t / p.tiles_per_row;
-    f0 = (t - row * p.tiles_per_row) * 32;
-    return t < p.total_tiles;
-  };
-  int64_t row, f0;
-  for (int64_t n = 0; n < 2; ++n)  // prologue: two tiles in flight
-    if (tile_of(n, row, f0)) r3_fill(p, row, f0, s_x + (size_t)(n % 3) * p.slot_floats, s_full + (n % 3), crank, tid, blockDim.x);
-  __syncthreads();
-  for (int64_t n = 0; tile_of(n, row, f0); ++n) {
-    const int slot = (int)(n % 3);
-    {  // stage tile n + 2 into the slot tile n - 1 used: every CTA of the cluster must have released it
-      int64_t nrow, nf0;
-      if (tile_of(n + 2, nrow, nf0)) {
-        const int ns = (int)((n + 2) % 3);
-        if (n + 2 >= 3 && tid == 0) mbar_wait_cluster(s_empty + ns, (uint32_t)(((n + 2) / 3 - 1) & 1));
-        __syncthreads();  // (the local scalar part may be written now too)
-        asm volatile("fence.proxy.async.shared::cta;" ::: "memory");
-        r3_fill(p, nrow, nf0, s_x + (size_t)ns * p.slot_floats, s_full + ns, crank, tid, blockDim.x);
-      }
-    }
-    mbar_wait_cluster(s_full + slot, (uint32_t)((n / 3) & 1));
-    if (active) {
-      const float* xs = s_x + (size_t)slot * p.slot_floats + r3_shift(p, row, f0) + lane * p.orig_r + qb;
-      uint64_t a01e = 0ull, a23e = 0ull, a01o = 0ull, a23o = 0ull;
-#pragma unroll
-      for (int i = 0; i < kR3Len; i += 2) {
-        const float x0 = xs[i], x1 = xs[i + 1];
-        a01e = fma2_raw(pk2(tp[i].x, tp[i].y), pk2(x0, x0), a01e);
-        a23e = fma2_raw(pk2(tp[i].z, tp[i].w), pk2(x0, x0), a23e);
-        a01o = fma2_raw(pk2(tp[i + 1].x, tp[i + 1].y), pk2(x1, x1), a01o);
-        a23o = fma2_raw(pk2(tp[i + 1].z, tp[i + 1].w), pk2(x1, x1), a23o);
-      }
-      const float2 y01 = upk2(add2_raw(a01e, a01o)), y23 = upk2(add2_raw(a23e, a23o));
-      const int64_t f = f0 + lane;
-      if (f < p.frames) {
-        const int64_t n0 = f * p.new_r + j0;
-        float* o = p.out + row * p.out_row_stride + n0;
-        if (p.out_vec && j0 + 4 <= p.new_r && n0 + 4 <= p.out_len) {
-          *reinterpret_cast<float4*>(o) = make_float4(y01.x, y01.y, y23.x, y23.y);
-        } else {
-          const float y[4] = {y01.x, y01.y, y23.x, y23.y};
-#pragma unroll
-          for (int r = 0; r < 4; ++r)
-            if (j0 + r < p.new_r && n0 + r < p.out_len) o[r] = y[r];
-        }
-      }
-    }
-    __syncthreads();  // this CTA is done with the slot ...
-    if (tid == 0)     // ... tell every CTA of the cluster (they multicast into it)
-      for (uint32_t r = 0; r < (uint32_t)p.csize; ++r) mbar_arrive_remote(s_empty + slot, r);
-  }
-  cluster_sync_all();  // nobody leaves while a peer may still arrive on its barriers
 }
 
 // Straightforward one-output-per-thread kernel (any ratio).  Consecutive threads are consecutive
@@ -945,8 +392,8 @@ resample_direct_kernel(const float* __restrict__ wave, int64_t length, int64_t r
 //   One thread issues, per 16-tap k-step, TWO tcgen05.mma (taps_hi, taps_lo accumulate into the same columns) whose
 //   B operand holds only the phases that have live taps in that step, banded like the mel filterbank: 60 instructions
 //   of N = 8..32 per tile instead of 960 legacy HMMAs.  The accumulator (<= 160 columns) is double buffered in tensor
-//   memory; eight epilogue warps (two per TMEM lane quadrant, half the columns each) read it (tcgen05.ld), add the
-//   hi / lo ROWS of a frame with one shuffle and store 64 bytes per thread.
+//   memory; four epilogue warps (one per TMEM lane quadrant) read it (tcgen05.ld), add the hi / lo ROWS of a frame
+//   with one shuffle and store 64 bytes per thread.
 //   Shared memory at 441:160: 2 x 60 KB operand + 43 KB taps + 4 x 14 KB staged; HBM traffic = the algorithmic bytes.
 //   Arithmetic: bf16 x 3 (x_hi k_hi + x_hi k_lo + x_lo k_hi + x_lo k_lo), FP32 accumulate: ~5e-6 of the peak.
 // ================================================================================================
@@ -961,21 +408,11 @@ constexpr int kTcAStride = 1024;       // bytes per 8-tap chunk: 8 row groups x 
 // instructions of a tile took 6100 cycles instead of 1800.
 //   warps 0-3 epilogue (TMEM lane quadrant = warp), 7 issuer, 11 producer, the other warps with warp % 4 != 3 convert
 //   (12 of them); warp 15 has no role
-#ifndef B200A_TC_EPI
-#define B200A_TC_EPI 4
-#endif
-#ifndef B200A_TC_PACKED_SHFL
-#define B200A_TC_PACKED_SHFL 0  // measured: 5 % fewer L1TEX cycles, no time gained, 2.3x the rounding error
-#endif
-constexpr int kTcConvWarps = 12, kTcEpiWarps = B200A_TC_EPI;  // 4: one per TMEM lane quadrant; 8: two, half the columns each
+constexpr int kTcConvWarps = 12, kTcEpiWarps = 4;  // one epilogue warp per TMEM lane quadrant
 constexpr int kTcWarps = kTcEpiWarps + 15;
 constexpr int kTcThreads = kTcWarps * 32;
 constexpr int kTcIssuerWarp = kTcEpiWarps + 3, kTcProducerWarp = kTcEpiWarps + 7;
-#ifndef B200A_TC_PREFETCH
-#define B200A_TC_PREFETCH 0
-#endif
-constexpr int kTcPrefetchTiles = B200A_TC_PREFETCH;  // tiles pulled into L2 ahead of the staged one (measured: no gain)
-constexpr int kTcMaxPhases = 160;      // columns of one accumulator
+constexpr int kTcMaxPhases = 160;     // columns of one accumulator
 constexpr int kTcAccStride = 256;      // TMEM columns between the two accumulators
 constexpr int kTcSmemLimit = 227 * 1024;
 constexpr int kTcIssueBytes = 2 * (2 * kTcMaxKSteps + 2) * 16;  // per accumulator / operand buffer: one uint4 per MMA
@@ -1121,7 +558,6 @@ __global__ void resample_tc_plan_kernel(const float* __restrict__ kernel, const 
 }
 
 struct RsTcParams {
-  long long* trace;  // B200A_TC_TRACE builds: [16 tiles][16 events] clock64 stamps of CTA 0 (else unused)
   const float* wave;
   int64_t rows, length, row_stride;
   float* out;
@@ -1149,16 +585,9 @@ __device__ __forceinline__ void tmem_ld_pin(float (&v)[16]) {
                : "memory");
 }
 
-#ifdef B200A_TC_TRACE
-#define TC_STAMP(n, ev) do { if (blockIdx.x == 0 && (n) < 16 && lane == 0 && p.trace) p.trace[(n) * 16 + (ev)] = clock64(); } while (0)
-#else
-#define TC_STAMP(n, ev) do { } while (0)
-#endif
-
-__global__ void __launch_bounds__(kTcThreads, 1) resample_tc_kernel(const RsTcParams p, const __grid_constant__ RsTcIssueTab tab,
-                                                                    int require_flag) {
+__global__ void __launch_bounds__(kTcThreads, 1) resample_tc_kernel(const RsTcParams p, const __grid_constant__ RsTcIssueTab tab) {
   extern __shared__ __align__(128) unsigned char smem_raw[];
-  if (require_flag && p.hdr->tc_ok == 0) return;  // (uniform) the mma.sync kernel launched next does the work
+  if (p.hdr->tc_ok == 0) return;  // (uniform) the mma.sync kernel launched next does the work
   const RsTcSmem m = rs_tc_smem(p.orig_r, p.taps);
   unsigned char* s_a = smem_raw;                                              // [2][n_chunks][1024]
   unsigned char* s_zero = smem_raw + m.zero_off;                              // [2][1024]
@@ -1232,56 +661,34 @@ __global__ void __launch_bounds__(kTcThreads, 1) resample_tc_kernel(const RsTcPa
   };
 
   if (warp < kTcEpiWarps) {
-    // ============ epilogue warps: TMEM lane quadrant warp % 4; with eight of them, column half warp / 4 ===========
-    const int cw = warp & 3, ch = warp >> 2;
-    const int split = kTcEpiWarps == 8 ? (n_pad / 32 + 1) / 2 * 32 : n_pad;  // whole 32-column passes: [0, split), [split, n_pad)
-    const int j_first = ch ? split : 0, j_last = ch ? n_pad : (split < n_pad ? split : n_pad);
+    // ============ epilogue warps: TMEM lane quadrant = warp ==========================================================
     int64_t row, f0;
     for (int n = 0; tile_of(n, row, f0); ++n) {
       const int b = n & 1;
-      if (warp == 0) TC_STAMP(n, 0);
       mbar_wait(s_mma + b, (uint32_t)(n >> 1) & 1u);
-      if (warp == 0) TC_STAMP(n, 1);
       tc_fence_after();
-      const uint32_t acc = tmem_d + ((uint32_t)(32 * cw) << 16) + (uint32_t)(b * kTcAccStride);
-      const int64_t f = f0 + 8 * cw + (lane & 7);  // lanes 0-7: hi rows of frames 8 cw .. 8 cw + 7, lanes 8-15: their lo rows
+      const uint32_t acc = tmem_d + ((uint32_t)(32 * warp) << 16) + (uint32_t)(b * kTcAccStride);
+      const int64_t f = f0 + 8 * warp + (lane & 7);  // lanes 0-7: hi rows of frames 8 warp .. + 7, lanes 8-15: their lo rows
       const bool own = lane < 8 && f < p.frames;
       float* orow = p.out + row * p.out_row_stride + f * p.new_r;
       const int64_t n0 = f * p.new_r;
-      auto store16 = [&](int j, const float (&y)[16]) {
-        if (p.out_vec && j + 16 <= j_last && j + 16 <= p.new_r && n0 + j + 16 <= p.out_len) {
+      auto store16 = [&](int j, const float (&y)[16]) {  // (j < n_pad follows from j < new'; ptxas uses 1 register less with it)
+        if (p.out_vec && j + 16 <= n_pad && j + 16 <= p.new_r && n0 + j + 16 <= p.out_len) {
 #pragma unroll
           for (int q = 0; q < 16; q += 4)
             *reinterpret_cast<float4*>(orow + j + q) = make_float4(y[q], y[q + 1], y[q + 2], y[q + 3]);
         } else {
 #pragma unroll
           for (int q = 0; q < 16; ++q)
-            if (j + q < j_last && j + q < p.new_r && n0 + j + q < p.out_len) orow[j + q] = y[q];
+            if (j + q < n_pad && j + q < p.new_r && n0 + j + q < p.out_len) orow[j + q] = y[q];
         }
       };
       auto finish32 = [&](int j, float (&u)[16], float (&w)[16]) {
-#if B200A_TC_PACKED_SHFL
-        // x_hi row + x_lo row.  The x_lo row is a 2^-9 correction: it crosses the lanes as bf16 pairs (2^-18 of the
-        // result), which halves the shuffles -- the shared-memory / shuffle pipe is the busiest unit of this kernel.
-#pragma unroll
-        for (int q = 0; q < 16; q += 2) {
-          uint32_t pu, pw;
-          asm("cvt.rn.bf16x2.f32 %0, %1, %2;" : "=r"(pu) : "f"(u[q + 1]), "f"(u[q]));
-          asm("cvt.rn.bf16x2.f32 %0, %1, %2;" : "=r"(pw) : "f"(w[q + 1]), "f"(w[q]));
-          pu = __shfl_down_sync(0xffffffffu, pu, 8);
-          pw = __shfl_down_sync(0xffffffffu, pw, 8);
-          u[q] += __uint_as_float(pu << 16);
-          u[q + 1] += __uint_as_float(pu & 0xffff0000u);
-          w[q] += __uint_as_float(pw << 16);
-          w[q + 1] += __uint_as_float(pw & 0xffff0000u);
-        }
-#else
 #pragma unroll
         for (int q = 0; q < 16; ++q) {
           u[q] += __shfl_down_sync(0xffffffffu, u[q], 8);  // x_hi row + x_lo row
           w[q] += __shfl_down_sync(0xffffffffu, w[q], 8);
         }
-#endif
         if (own) {
           store16(j, u);
           store16(j + 16, w);
@@ -1289,23 +696,23 @@ __global__ void __launch_bounds__(kTcThreads, 1) resample_tc_kernel(const RsTcPa
       };
       // two register sets: the tensor-memory load of the next 32 columns is in flight while these are summed and stored
       float ua[16], wa[16], ub[16], wb[16];
-      tmem_ld16_nowait(acc + j_first, ua);
-      tmem_ld16_nowait(acc + j_first + 16, wa);  // (columns past n_pad: allocated, never stored)
+      tmem_ld16_nowait(acc, ua);
+      tmem_ld16_nowait(acc + 16, wa);  // (columns past n_pad: allocated, never stored)
 #pragma unroll 1
-      for (int j0 = j_first; j0 < j_last; j0 += 64) {
+      for (int j0 = 0; j0 < n_pad; j0 += 64) {
         asm volatile("tcgen05.wait::ld.sync.aligned;" ::: "memory");
         tmem_ld_pin(ua);
         tmem_ld_pin(wa);
-        if (j0 + 32 < j_last) {
+        if (j0 + 32 < n_pad) {
           tmem_ld16_nowait(acc + j0 + 32, ub);
           tmem_ld16_nowait(acc + j0 + 48, wb);
         }
         finish32(j0, ua, wa);
-        if (j0 + 32 < j_last) {
+        if (j0 + 32 < n_pad) {
           asm volatile("tcgen05.wait::ld.sync.aligned;" ::: "memory");
           tmem_ld_pin(ub);
           tmem_ld_pin(wb);
-          if (j0 + 64 < j_last) {
+          if (j0 + 64 < n_pad) {
             tmem_ld16_nowait(acc + j0 + 64, ua);
             tmem_ld16_nowait(acc + j0 + 80, wa);
           }
@@ -1314,7 +721,6 @@ __global__ void __launch_bounds__(kTcThreads, 1) resample_tc_kernel(const RsTcPa
       }
       tc_fence_before();
       __syncwarp();
-      if (warp == 0) TC_STAMP(n, 2);
       if (lane == 0) mbar_arrive(s_accfree + b);
     }
     tc_fence_before();
@@ -1329,9 +735,7 @@ __global__ void __launch_bounds__(kTcThreads, 1) resample_tc_kernel(const RsTcPa
       const int b = n & 1;
       const uint4* rec = s_issue + b * (2 * kTcMaxKSteps + 2);
       mbar_wait(s_aready + b, (uint32_t)(n >> 1) & 1u);  // every convert warp is through with the tile: operand complete
-      TC_STAMP(n, 10);
       if (n >= 2) mbar_wait(s_accfree + b, (uint32_t)((n >> 1) - 1) & 1u);  // tile n - 2 has left this accumulator
-      TC_STAMP(n, 11);
       tc_fence_after();
       if (leader) {
         {
@@ -1346,7 +750,6 @@ __global__ void __launch_bounds__(kTcThreads, 1) resample_tc_kernel(const RsTcPa
         umma_commit(s_mma + b);
       }
       __syncwarp();
-      TC_STAMP(n, 12);
     }
   } else if (warp == kTcProducerWarp) {
     // ============ producer warp: unit u of tile n + 1 follows unit u of tile n into slot u ==========================
@@ -1396,28 +799,12 @@ __global__ void __launch_bounds__(kTcThreads, 1) resample_tc_kernel(const RsTcPa
         }
       }
     };
-    // Shared memory holds one tile of samples (57 KB per SM, 8 MB over the GPU): less than HBM latency x bandwidth,
-    // so the tiles after the staged one are pulled into L2 ahead of time.
-    auto prefetch_tile = [&](int n) {
-      int64_t row, f0;
-      if (kTcPrefetchTiles == 0 || !tile_of(n, row, f0)) return;
-      const float* x = p.wave + row * p.row_stride;
-      const int64_t T0 = f0 * p.orig_r - p.width;
-      int64_t lo = T0 < 0 ? 0 : T0, hi = T0 + (int64_t)(kTcFrames - 1) * p.orig_r + 8 * n_chunks;
-      if (hi > p.length) hi = p.length;
-      lo += (4 - ((reinterpret_cast<uintptr_t>(x + lo) >> 2) & 3)) & 3;  // 16-byte aligned start, whole 16-byte pieces
-      const int64_t cnt = (hi - lo) & ~(int64_t)3;
-      if (lane == 0 && cnt > 0) bulk_prefetch_l2(x + lo, (uint32_t)cnt * 4u);
-    };
     for (int u = 0; u < kTcUnits; ++u) stage_unit(0, u);
-    for (int d = 1; d <= kTcPrefetchTiles; ++d) prefetch_tile(d);
     int64_t row, f0;
     for (int n = 0; tile_of(n, row, f0); ++n) {
-      prefetch_tile(n + 1 + kTcPrefetchTiles);
 #pragma unroll 1
       for (int u = 0; u < kTcUnits; ++u) {
         mbar_wait(s_cdone + u, (uint32_t)n & 1u);
-        if (u == 0) TC_STAMP(n, 9);
         stage_unit(n + 1, u);
       }
     }
@@ -1430,15 +817,12 @@ __global__ void __launch_bounds__(kTcThreads, 1) resample_tc_kernel(const RsTcPa
     int64_t row, f0;
     for (int n = 0; tile_of(n, row, f0); ++n) {
       const int b = n & 1;
-      if (cv == 0) TC_STAMP(n, 3);
       if (n >= 2) mbar_wait(s_mma + b, (uint32_t)((n >> 1) - 1) & 1u);  // tile n - 2 has been multiplied: operand b is free
-      if (cv == 0) TC_STAMP(n, 4);
       unsigned char* abuf = s_a + b * m.a_bytes;
       int it = cv;  // items of the tile in unit order, dealt round robin: g = u ipu + it belongs to warp g % kTcConvWarps
 #pragma unroll 1
       for (int u = 0; u < kTcUnits; ++u) {
         mbar_wait(s_full + u, (uint32_t)n & 1u);  // the unit's samples are staged (every warp waits, items or not)
-        if (cv == 0 && u == 0) TC_STAMP(n, 5);
         const float* xs = s_x + u * m.slot_floats + s_shift[u] + lane_off;  // this frame's tap 0
         // frame F = 8 u + fl: hi row in group 2 u, row fl; the lo row 128 bytes on
         unsigned char* arow = abuf + u * 256 + fl * 16;
@@ -1464,10 +848,36 @@ __global__ void __launch_bounds__(kTcThreads, 1) resample_tc_kernel(const RsTcPa
       }
       asm volatile("fence.proxy.async.shared::cta;" ::: "memory");  // my operand rows -> the tensor core
       __syncwarp();
-      if (cv == 0) TC_STAMP(n, 6);
       if (lane == 0) mbar_arrive(s_aready + b);
     }
   }
+}
+
+// The kernel family of a ratio, from (orig', new', width) alone: resample_plan_info_impl reports it and
+// resample_run_impl launches it (after the per-call conditions only a run can check).  Never chosen by the batch, so
+// a row's result does not depend on what it is batched with.
+enum RsFamily { kRsFamilyTc = 1, kRsFamilyMma = 2, kRsFamilyDirect = 3 };  // b200a_resample_plan_info info[0]
+struct RsChoice {
+  int family;
+  RsTcSteps tc;       // the banded tcgen05 plan (tc.ok: it fits)
+  int n_tiles;        // mma.sync kernel: groups of 8 phases,
+  int xs_floats;      // floats per staging buffer,
+  size_t smem_fixed;  // and its shared memory before the fragment copy
+};
+inline RsChoice rs_choose(int orig_r, int new_r, int width) {
+  RsChoice c{};
+  const int taps = 2 * width + orig_r;
+  c.tc = rs_tc_steps(orig_r, new_r, width);
+  c.n_tiles = rs_tiles(new_r);
+  c.xs_floats = (kRsFrames * orig_r + taps + 16 + 4 + 3) & ~3;  // rs_fill's span + its alignment shift, whole float4
+  c.smem_fixed = sizeof(float) * 2 * (size_t)c.xs_floats + 16 + sizeof(RsTile) * ((c.n_tiles + 3) & ~3);
+  const bool mma = c.n_tiles <= kRsMaxTiles && c.smem_fixed + 1024 <= (size_t)kRsSmemBudget;
+  // tcgen05 for odd orig' (conflict-free frame-per-lane reads) whenever its plan fits: 0.283 vs 0.391 ms at config 3,
+  // bf16 x 3 arithmetic (~6e-6 of the output peak against ~1e-6 for TF32 x 3).  The mma.sync kernel runs behind it as
+  // the device-side fallback, so it must fit too (within the tcgen05 limits it always does).
+  const bool tc = (orig_r & 1) != 0 && c.tc.ok != 0;
+  c.family = !mma ? kRsFamilyDirect : (tc ? kRsFamilyTc : kRsFamilyMma);
+  return c;
 }
 
 }  // namespace
@@ -1480,18 +890,11 @@ size_t resample_workspace_bytes_impl(int new_r, int taps) { return rs_layout(new
 //   info[2] dynamic shared memory of the tcgen05 kernel, info[3] its MMAs per 32-frame tile
 int resample_plan_info_impl(int orig_r, int new_r, int width, int32_t* info) {
   if (orig_r < 1 || new_r < 1 || width < 0 || info == nullptr) return B200A_EINVAL;
-  const int taps = 2 * width + orig_r;
-  const RsTcSteps steps = rs_tc_steps(orig_r, new_r, width);
-  const RsTcSmem tcm = rs_tc_smem(orig_r, taps);
-  const bool tc = (orig_r & 1) != 0 && steps.ok != 0;
-  const int n_tiles = rs_tiles(new_r);
-  const int xs_floats = (kRsFrames * orig_r + taps + 16 + 4 + 3) & ~3;
-  const size_t smem_fixed = sizeof(float) * 2 * (size_t)xs_floats + 16 + sizeof(RsTile) * ((n_tiles + 3) & ~3);
-  const bool mma = n_tiles <= kRsMaxTiles && smem_fixed + 1024 <= (size_t)kRsSmemBudget;
-  info[0] = tc ? 1 : (mma ? 2 : 3);
-  info[1] = steps.ok ? steps.b_bytes : 0;
-  info[2] = steps.ok ? tcm.total : 0;
-  info[3] = steps.ok ? 2 * steps.steps + 1 : 0;
+  const RsChoice c = rs_choose(orig_r, new_r, width);
+  info[0] = c.family;
+  info[1] = c.tc.ok ? c.tc.b_bytes : 0;
+  info[2] = c.tc.ok ? rs_tc_smem(orig_r, 2 * width + orig_r).total : 0;
+  info[3] = c.tc.ok ? 2 * c.tc.steps + 1 : 0;
   return B200A_OK;
 }
 
@@ -1521,16 +924,9 @@ int resample_prepare_impl(const float* kernel, int orig_r, int new_r, int width,
   if (rs_tiles(new_r) <= kRsMaxTiles)
     resample_plan_kernel<<<1, 256, 0, stream>>>(kernel, support, new_r, taps, rs_tiles(new_r), hdr,
                                                 reinterpret_cast<RsTile*>(base + l.tiles),
-                                                reinterpret_cast<float4*>(base + l.frags),
-                                                reinterpret_cast<uint4*>(base + l.frags16));
-  resample_r3_plan_kernel<<<1, 256, 0, stream>>>(kernel, support, new_r, taps, (new_r + 3) / 4, hdr,
-                                                 reinterpret_cast<int*>(base + l.r3base),
-                                                 reinterpret_cast<float4*>(base + l.r3taps));
+                                                reinterpret_cast<float4*>(base + l.frags));
   resample_tc_plan_kernel<<<1, 256, 0, stream>>>(kernel, support, orig_r, new_r, width, taps,
                                                  rs_tc_steps(orig_r, new_r, width), hdr, base + l.tcblocks);
-  resample_simt_plan_kernel<<<1, 256, 0, stream>>>(kernel, support, new_r, taps, rs_tiles(new_r), hdr,
-                                                   reinterpret_cast<RsSimtGroup*>(base + l.sgroups),
-                                                   reinterpret_cast<float*>(base + l.staps));
   return launch_status();
 }
 
@@ -1543,200 +939,47 @@ int resample_run_impl(const void* ws, const float* kernel, int orig_r, int new_r
   const int taps = 2 * width + orig_r;
   const RsLayout l = rs_layout(new_r, taps);
   const unsigned char* base = static_cast<const unsigned char*>(ws);
-
-  // B200A_RS=tc|simt|mma|bf16|direct|r3 forces one kernel family (A/B measurements, tests); default: the first that applies
-  static const int forced = [] {
-    const char* e = std::getenv("B200A_RS");
-    if (e == nullptr) return 0;
-    return e[0] == 's' ? 1 : (e[0] == 'm' ? 2 : (e[0] == 'd' ? 3 : (e[0] == 'b' ? 4 : (e[0] == 'r' ? 5 : (e[0] == 't' ? 6 : 0)))));
-  }();
+  const RsChoice c = rs_choose(orig_r, new_r, width);
+  // per call: the bulk copies of both tensor-core kernels need a 4-byte aligned input (rows may have any pitch), and
+  // the tcgen05 kernel takes rows shorter than 2^31 samples (with a tile's margin); longer rows go to mma.sync
+  const bool aligned = (reinterpret_cast<uintptr_t>(wave) & 3) == 0;
   int dev = 0, sms = 0;
   if (cudaGetDevice(&dev) != cudaSuccess || cudaDeviceGetAttribute(&sms, cudaDevAttrMultiProcessorCount, dev) != cudaSuccess)
     return B200A_ECUDA;
 
-  // ---- cluster path: taps in registers, tiles multicast to the CTAs that share the phases --------------------------
-  bool r3_launched = false;
-  {
-    const int n_quads = (new_r + 3) / 4;
-    const int csize = (n_quads + kR3Warps - 1) / kR3Warps;  // CTAs that share a tile: 5 at 441:160
-    const int slot_floats = (32 * orig_r + 2 * width + 16 + 3 + 3 + kR3Len) & ~3;
-    const size_t smem = sizeof(float) * 3 * (size_t)slot_floats + 64;
-    const bool want = forced == 5;  // measured 1.80 ms at config 3 (cluster-scope barrier latency per 32-frame tile): opt-in only
-    if (want && csize <= kR3MaxCluster && smem <= (size_t)227 * 1024 && (reinterpret_cast<uintptr_t>(wave) & 3) == 0 &&
-        length + (int64_t)taps + 64 * (int64_t)orig_r < ((int64_t)1 << 31)) {
-      R3Params p{};
-      p.wave = wave;
-      p.rows = rows;
-      p.length = length;
-      p.row_stride = row_stride;
-      p.out = out;
-      p.out_row_stride = out_row_stride;
-      p.out_len = out_len;
-      p.hdr = reinterpret_cast<const RsHeader*>(base + l.header);
-      p.qbase = reinterpret_cast<const int*>(base + l.r3base);
-      p.qtaps = reinterpret_cast<const float4*>(base + l.r3taps);
-      p.orig_r = orig_r;
-      p.new_r = new_r;
-      p.width = width;
-      p.n_quads = n_quads;
-      p.csize = csize;
-      p.frames = (out_len + new_r - 1) / new_r;
-      p.tiles_per_row = (p.frames + 31) / 32;
-      p.total_tiles = rows * p.tiles_per_row;
-      p.out_vec = (new_r % 4 == 0 && out_row_stride % 4 == 0 && (reinterpret_cast<uintptr_t>(out) & 15) == 0) ? 1 : 0;
-      if (cudaFuncSetAttribute(resample_r3_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, 227 * 1024) != cudaSuccess)
-        return B200A_ECUDA;
-      cudaLaunchConfig_t cfg{};
-      cudaLaunchAttribute attr[1];
-      attr[0].id = cudaLaunchAttributeClusterDimension;
-      attr[0].val.clusterDim.x = (unsigned)csize;
-      attr[0].val.clusterDim.y = 1;
-      attr[0].val.clusterDim.z = 1;
-      cfg.blockDim = dim3(kR3Warps * 32, 1, 1);
-      cfg.dynamicSmemBytes = smem;
-      cfg.stream = stream;
-      cfg.attrs = attr;
-      cfg.numAttrs = 1;
-      cfg.gridDim = dim3((unsigned)csize, 1, 1);
-      int max_clusters = 0;
-      const cudaError_t occ = cudaOccupancyMaxActiveClusters(&max_clusters, resample_r3_kernel, &cfg);
-      if (std::getenv("B200A_DEBUG") != nullptr)
-        std::fprintf(stderr, "[b200a] r3: csize=%d smem=%zu occupancy query: %s, max_clusters=%d\n", csize, smem,
-                     cudaGetErrorString(occ), max_clusters);
-      if (occ == cudaSuccess && max_clusters > 0) {
-        int64_t n_clusters = p.total_tiles < max_clusters ? p.total_tiles : max_clusters;
-        if (n_clusters < 1) n_clusters = 1;
-        cfg.gridDim = dim3((unsigned)(n_clusters * csize), 1, 1);
-        const int require_flag = forced == 5 ? 0 : 1;
-        const cudaError_t le = cudaLaunchKernelEx(&cfg, resample_r3_kernel, p, require_flag);
-        if (std::getenv("B200A_DEBUG") != nullptr)
-          std::fprintf(stderr, "[b200a] r3: launch %u CTAs: %s\n", cfg.gridDim.x, cudaGetErrorString(le));
-        if (le != cudaSuccess) return B200A_ECUDA;
-        if (forced == 5) return launch_status();
-        r3_launched = true;  // the tensor-pipe kernel below runs only if the plan says the quads did not fit
-      } else {
-        (void)cudaGetLastError();
-      }
-    }
-    if (forced == 5 && !r3_launched) return B200A_EUNSUPPORTED;
-  }
-
   // ---- tcgen05 path: banded bf16 x 3 product, operand built in shared memory per 32-frame tile --------------------
   bool tc_launched = false;
-  {
+  if (c.family == kRsFamilyTc && aligned && length + (int64_t)taps + 64 * (int64_t)orig_r < ((int64_t)1 << 31)) {
     const RsTcSmem tcm = rs_tc_smem(orig_r, taps);
-    const size_t smem = (size_t)tcm.total;
-    // default for odd orig' (conflict-free frame-per-lane reads) whenever the plan fits: 0.283 vs 0.391 ms at config 3.
-    // Chosen by the RATIO alone, never by the batch, so that a row's result does not depend on what it is batched with.
-    // bf16 x 3 arithmetic: ~6e-6 of the output peak against ~1e-6 for the TF32 x 3 kernel below.
-    const bool want = forced == 6 || (forced == 0 && (orig_r & 1) != 0);
-    const RsTcSteps steps = rs_tc_steps(orig_r, new_r, width);
-    if (want && steps.ok &&
-        (reinterpret_cast<uintptr_t>(wave) & 3) == 0 && length + (int64_t)taps + 64 * (int64_t)orig_r < ((int64_t)1 << 31)) {
-      RsTcParams p{};
-      p.wave = wave;
-      p.rows = rows;
-      p.length = length;
-      p.row_stride = row_stride;
-      p.out = out;
-      p.out_row_stride = out_row_stride;
-      p.out_len = out_len;
-      p.hdr = reinterpret_cast<const RsHeader*>(base + l.header);
-      p.blocks = base + l.tcblocks;
-      p.orig_r = orig_r;
-      p.new_r = new_r;
-      p.width = width;
-      p.taps = taps;
-      p.frames = (out_len + new_r - 1) / new_r;
-      p.tiles_per_row = (p.frames + kTcFrames - 1) / kTcFrames;
-      p.total_tiles = rows * p.tiles_per_row;
-      p.out_vec = (new_r % 4 == 0 && out_row_stride % 4 == 0 && (reinterpret_cast<uintptr_t>(out) & 15) == 0) ? 1 : 0;
-      if (cudaFuncSetAttribute(resample_tc_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, 227 * 1024) != cudaSuccess)
-        return B200A_ECUDA;
-      int64_t grid = p.total_tiles < sms ? p.total_tiles : sms;
-      if (grid < 1) grid = 1;
-#ifdef B200A_TC_TRACE
-      static long long* trace_dev = nullptr;
-      if (trace_dev == nullptr) cudaMalloc(&trace_dev, sizeof(long long) * 256);
-      cudaMemsetAsync(trace_dev, 0, sizeof(long long) * 256, stream);
-      p.trace = trace_dev;
-#endif
-      resample_tc_kernel<<<(unsigned)grid, kTcThreads, smem, stream>>>(p, rs_tc_issue_tab(steps, tcm.n_chunks), 1);
-#ifdef B200A_TC_TRACE
-      {
-        long long h[256];
-        cudaStreamSynchronize(stream);
-        cudaMemcpy(h, trace_dev, sizeof(h), cudaMemcpyDeviceToHost);
-        static int shown = 0;
-        if (shown++ == 3) {
-          const long long t0 = h[3];
-          std::fprintf(stderr, "[tc trace] tile: epi(wait got done) conv(start full loFree hiFree done) - prod(cd0) issue(alo accfree issued)\n");
-          for (int n = 0; n < 16; ++n) {
-            std::fprintf(stderr, "[tc trace] %2d:", n);
-            for (int e = 0; e < 13; ++e) std::fprintf(stderr, " %7lld", h[n * 16 + e] ? h[n * 16 + e] - t0 : -1);
-            std::fprintf(stderr, "\n");
-          }
-        }
-      }
-#endif
-      if (cudaPeekAtLastError() != cudaSuccess) return launch_status();
-      tc_launched = true;  // the mma.sync kernel below runs only if the device-side plan did not fit
-    }
+    RsTcParams p{};
+    p.wave = wave;
+    p.rows = rows;
+    p.length = length;
+    p.row_stride = row_stride;
+    p.out = out;
+    p.out_row_stride = out_row_stride;
+    p.out_len = out_len;
+    p.hdr = reinterpret_cast<const RsHeader*>(base + l.header);
+    p.blocks = base + l.tcblocks;
+    p.orig_r = orig_r;
+    p.new_r = new_r;
+    p.width = width;
+    p.taps = taps;
+    p.frames = (out_len + new_r - 1) / new_r;
+    p.tiles_per_row = (p.frames + kTcFrames - 1) / kTcFrames;
+    p.total_tiles = rows * p.tiles_per_row;
+    p.out_vec = (new_r % 4 == 0 && out_row_stride % 4 == 0 && (reinterpret_cast<uintptr_t>(out) & 15) == 0) ? 1 : 0;
+    if (cudaFuncSetAttribute(resample_tc_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, 227 * 1024) != cudaSuccess)
+      return B200A_ECUDA;
+    int64_t grid = p.total_tiles < sms ? p.total_tiles : sms;
+    if (grid < 1) grid = 1;
+    resample_tc_kernel<<<(unsigned)grid, kTcThreads, (size_t)tcm.total, stream>>>(p, rs_tc_issue_tab(c.tc, tcm.n_chunks));
+    if (cudaPeekAtLastError() != cudaSuccess) return launch_status();
+    tc_launched = true;  // the mma.sync kernel below runs only if the device-side plan did not fit
   }
 
-  // ---- packed-FP32 SIMT path: odd orig' (conflict-free frame-per-lane reads) and the 3-slot ring fits -------------
-  {
-    const int n_groups = rs_tiles(new_r);
-    const int slot_floats = (32 * orig_r + 2 * width + 3 + 8 + 3) & ~3;  // span + alignment shift + zero-tap over-read
-    const size_t ring_bytes = sizeof(float) * 3 * (size_t)slot_floats;
-    const size_t fixed = ring_bytes + sizeof(RsSimtGroup) * (size_t)n_groups + 64;
-    const bool want = forced == 1;  // measured slower than the tensor-pipe kernel (0.446 vs 0.391 ms at config 3): opt-in only
-    if (want && fixed + 8192 <= (size_t)227 * 1024 && (reinterpret_cast<uintptr_t>(wave) & 3) == 0 &&
-        length + (int64_t)taps + 64 * (int64_t)orig_r < ((int64_t)1 << 31)) {
-      RsSimtParams p{};
-      p.wave = wave;
-      p.rows = rows;
-      p.length = length;
-      p.row_stride = row_stride;
-      p.out = out;
-      p.out_row_stride = out_row_stride;
-      p.out_len = out_len;
-      p.hdr = reinterpret_cast<const RsHeader*>(base + l.header);
-      p.groups = reinterpret_cast<const RsSimtGroup*>(base + l.sgroups);
-      p.table = reinterpret_cast<const float*>(base + l.staps);
-      p.orig_r = orig_r;
-      p.new_r = new_r;
-      p.width = width;
-      p.n_groups = n_groups;
-      p.frames = (out_len + new_r - 1) / new_r;
-      p.halves = (p.frames + 31) / 32;
-      p.total_halves = rows * p.halves;
-      p.out_vec = (new_r % 4 == 0 && out_row_stride % 4 == 0 && (reinterpret_cast<uintptr_t>(out) & 15) == 0) ? 1 : 0;
-      // the tap table gets whatever shared memory is left (the kernel compares the device-side size written by
-      // prepare with this room and reads the table through L1 instead when it does not fit)
-      const size_t tap_cap = sizeof(float) * 8 * (size_t)n_groups * ((size_t)taps + 8);
-      const size_t room = ((size_t)227 * 1024 - fixed) & ~(size_t)15;
-      p.tap_floats = (int)((tap_cap < room ? tap_cap : room) / sizeof(float));
-      const size_t smem = fixed + sizeof(float) * (size_t)p.tap_floats;
-      if (cudaFuncSetAttribute(resample_simt_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, 227 * 1024) != cudaSuccess)
-        return B200A_ECUDA;
-      int warps = (n_groups + 1) / 2;  // one phase group of the step's parity per warp
-      if (warps > kSimtMaxWarps) warps = kSimtMaxWarps;
-      if (warps < 4) warps = 4;
-      int64_t grid = p.total_halves < sms ? p.total_halves : sms;
-      if (grid < 1) grid = 1;
-      resample_simt_kernel<<<(unsigned)grid, warps * 32, smem, stream>>>(p);
-      return launch_status();
-    }
-    if (forced == 1) return B200A_EUNSUPPORTED;
-  }
-
-  // ---- tensor-pipe path -------------------------------------------------------------------------
-  const int n_tiles = rs_tiles(new_r);
-  const int xs_floats = (kRsFrames * orig_r + taps + 16 + 4 + 3) & ~3;
-  const size_t smem_fixed = sizeof(float) * 2 * (size_t)xs_floats + 16 + sizeof(RsTile) * ((n_tiles + 3) & ~3);
-  const bool aligned = (reinterpret_cast<uintptr_t>(wave) & 3) == 0;  // any float pointer; rows may have any pitch
-  if (forced != 3 && n_tiles <= kRsMaxTiles && aligned && smem_fixed + 1024 <= (size_t)kRsSmemBudget) {
+  // ---- mma.sync path (also the device-side fallback behind the tcgen05 kernel) -------------------
+  if (c.family != kRsFamilyDirect && aligned) {
     RsParams p{};
     p.wave = wave;
     p.rows = rows;
@@ -1748,24 +991,20 @@ int resample_run_impl(const void* ws, const float* kernel, int orig_r, int new_r
     p.hdr = reinterpret_cast<const RsHeader*>(base + l.header);
     p.tiles = reinterpret_cast<const RsTile*>(base + l.tiles);
     p.frags = reinterpret_cast<const float4*>(base + l.frags);
-    p.frags16 = reinterpret_cast<const uint4*>(base + l.frags16);
     p.orig_r = orig_r;
     p.new_r = new_r;
     p.width = width;
     p.taps = taps;
-    p.n_tiles = n_tiles;
+    p.n_tiles = c.n_tiles;
     p.frames = (out_len + new_r - 1) / new_r;
     p.blocks_per_row = (p.frames + kRsFrames - 1) / kRsFrames;
     p.total_blocks = rows * p.blocks_per_row;
-    p.xs_floats = xs_floats;
+    p.xs_floats = c.xs_floats;
     // fragments go to shared memory when they fit next to the staging buffers (the kernel compares the
     // device-side step count with the room granted here), otherwise they are read through L1
-    p.frag_smem_bytes = (int)(((size_t)kRsSmemBudget - smem_fixed) & ~(size_t)511);  // everything that is left
-    const size_t smem = smem_fixed + p.frag_smem_bytes;
-    // default: TF32 x 3 (2^-21 relative).  B200A_RS=bf16 selects the bf16 x 3 variant: measured 5 % faster at config 3
-    // (0.371 vs 0.391 ms) for 30x the rounding error, so it stays opt-in
-    auto kern = forced == 4 ? resample_mma_kernel<true> : resample_mma_kernel<false>;
-    if (cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, 227 * 1024) != cudaSuccess)
+    p.frag_smem_bytes = (int)(((size_t)kRsSmemBudget - c.smem_fixed) & ~(size_t)511);  // everything that is left
+    const size_t smem = c.smem_fixed + p.frag_smem_bytes;
+    if (cudaFuncSetAttribute(resample_mma_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, 227 * 1024) != cudaSuccess)
       return B200A_ECUDA;
     int64_t grid = p.total_blocks < sms ? p.total_blocks : sms;
     if (grid < 1) grid = 1;
@@ -1783,10 +1022,10 @@ int resample_run_impl(const void* ws, const float* kernel, int orig_r, int new_r
       if (worst < best_conf) { best_conf = worst; best_spread = spread; }
     }
     p.row_spread = best_spread;
-    p.skip_if_r3_ok = r3_launched ? 1 : (tc_launched ? 2 : 0);
+    p.behind_tc = tc_launched ? 1 : 0;
     p.out_pair = (new_r % 2 == 0 && out_row_stride % 2 == 0 && (reinterpret_cast<uintptr_t>(out) & 7) == 0) ? 1 : 0;
     // warps: n_tiles items (phase groups) per tile; prefer the largest count that divides them evenly
-    const int items = n_tiles;
+    const int items = c.n_tiles;
     int warps = 8;
     double best_idle = 2.0;
     for (int w = 8; w <= kRsMaxWarps; ++w) {
@@ -1794,7 +1033,7 @@ int resample_run_impl(const void* ws, const float* kernel, int orig_r, int new_r
       const double idle = 1.0 - (double)items / (double)(rounds * w);
       if (idle <= best_idle + 1e-9) { best_idle = idle; warps = w; }  // ties go to more warps
     }
-    kern<<<(unsigned)grid, warps * 32, smem, stream>>>(p);
+    resample_mma_kernel<<<(unsigned)grid, warps * 32, smem, stream>>>(p);
     return launch_status();
   }
 

@@ -539,7 +539,7 @@ def test_complex_pointers_need_8_byte_alignment(clib):
 # resampler: family per cell (host) and every cell guarded (device)
 # ---------------------------------------------------------------------------------------------------------------------
 TC, MMA, DIRECT = 1, 2, 3  # b200a_resample_plan_info info[0]
-kTcMaxPhases, kTcMaxKSteps, kRsMaxTiles = 160, 30, 128  # resample.cu: rs_tc_steps, resample_run_impl
+kTcMaxPhases, kTcMaxKSteps, kRsMaxTiles = 160, 30, 128  # resample.cu: rs_tc_steps, rs_choose
 KAISER_BEST = dict(lowpass_filter_width=64, rolloff=0.9475937167399596, resampling_method="sinc_interp_kaiser",
                    beta=14.769656459379492)
 KAISER_FAST = dict(lowpass_filter_width=16, rolloff=0.85, resampling_method="sinc_interp_kaiser", beta=8.555504641634386)

@@ -195,8 +195,8 @@ def test_config4_every_row_against_oracle_2d_and_3d():
 
 
 def test_config3_many_rows_against_oracle_and_mma_kernel():
-    """The packed-FP32 SIMT resampler streams half-chunks of several rows through one CTA: compare 256 full-length
-    rows with the oracle (not just the first two)."""
+    """At 44.1 -> 16 kHz the tcgen05 resampler walks the 32-frame tiles of several rows through one CTA: compare 256
+    full-length rows with the oracle (not just the first two)."""
     B, L = 256, 220500
     x = torch.randn(B, L, device=DEV, generator=torch.Generator(device=DEV).manual_seed(4321))
     r = T.Resample(44100, 16000, resampling_method="sinc_interp_kaiser").to(DEV)
